@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- batched MPC solve throughput of the B200 engine (and the CPU reference arm).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--problems B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--problems B] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its last timed step returned -- plan [H][2][B],
+losses [S][B] and best [B] (the winning start, as float32) -- to DIR/<name>.npy.  The inputs are seeded, so the same
+arguments give the same problems on every run and two builds can be compared output for output.  Above 64 MB in all
+a fixed, seeded sample of problems is written, with their indices in DIR/problem_index.npy.
 
 One step = one pass of the hot path over one batch: ONE ocd_solve_batch launch that runs
 NaivePlanner.generate_plan (3 starts x 100 SGD iterations + final losses + argmin) for B
@@ -37,9 +42,27 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True           # the bench writes nothing into the tree it runs from (it may be read-only)
 
 SHAPE = dict(H=5, C=2, L=3, S=3, n_iter=100)
 METRIC, UNIT = "mpc_solves_per_sec", "solves/s"
+DUMP_LIMIT = 64 * 10**6                  # bytes --dump-outputs may write, .npy headers included
+
+
+def dump_outputs(out_dir: str, out: dict, B: int) -> None:
+    """Writes one step's device outputs (problem axis last) as float32 .npy files under out_dir; above DUMP_LIMIT
+    a fixed, seeded sample of the problems, whose indices go to problem_index.npy (float64, exact)."""
+    host = {k: v.cpu().numpy() for k, v in out.items()}
+    host["best"] = host["best"].astype(np.float32)            # start indices 0..5: exact in float32
+    per_problem = sum(a.nbytes for a in host.values()) // B
+    if per_problem * B > DUMP_LIMIT - 4096:
+        n = (DUMP_LIMIT - 4096) // (per_problem + 8)          # + the float64 index of each kept problem
+        sel = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        host = {k: np.ascontiguousarray(a[..., sel]) for k, a in host.items()}
+        host["problem_index"] = sel.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 def _config(B, n_gpus, per_step=None):
@@ -178,7 +201,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--problems", type=int, default=1 << 20, help="MPC problems per GPU per step")
     ap.add_argument("--no-extras", action="store_true", help="skip e2e / cpu_baseline / cmaes legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -255,6 +284,8 @@ def main():
     ms_total = max_over_ranks(float(e0.elapsed_time(e1)))
     clocks = sampler.stop()
     launches = eng.kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sets[(W + K - 1) % NSETS][3], B)
     value = B * K * world_size / (ms_total * 1e-3)
     ms_per_step = ms_total / K
 

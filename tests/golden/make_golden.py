@@ -1,15 +1,15 @@
 #!/usr/bin/env python
 """Generate the golden vectors in tests/golden/*.json from the REFERENCE'S OWN PYTHON.
 
-Runs only in the build container (needs /root/reference; the GPU box has neither it nor
-this need -- the JSON files are committed).  The reference modules are imported unmodified
-from /root/reference; the TensorFlow primitives they call are supplied by the torch-backed
-stand-in in oracle/tf_shim (TensorFlow itself cannot be installed here -- see
+Needs a checkout of the reference (avikj/L4DC-MPC-OCD), which is not part of this repository:
+pass it as --reference DIR or in L4DC_REFERENCE_DIR.  The tests only read the committed JSON
+files.  The reference modules are imported unmodified from that checkout; the TensorFlow
+primitives they call are supplied by the torch-backed stand-in in oracle/tf_shim (see
 oracle/ocd_oracle.h "PARITY STATUS").  Nothing from this repo's oracle or engine is used to
 produce the numbers.
 
-    python tests/golden/make_golden.py --all --jobs 8      # ~15 min on 8 cores
-    python tests/golden/make_golden.py --part primitives   # one part
+    python tests/golden/make_golden.py --reference DIR --all --jobs 8      # ~15 min on 8 cores
+    python tests/golden/make_golden.py --reference DIR --part primitives   # one part
 
 Parts: primitives, features, mpc_reward, plans, planner_kats, and one episode_* part per
 (scenario, weights, variant).
@@ -28,15 +28,14 @@ from pathlib import Path
 
 HERE = Path(__file__).resolve().parent
 REPO = HERE.parent.parent
-REF = Path("/root/reference")
 
 
-def _setup_reference_imports():
-    if not REF.exists():
-        raise SystemExit("make_golden.py needs /root/reference (build container only)")
+def _setup_reference_imports(ref: Path):
+    if not (ref / "interact_drive").is_dir():
+        raise SystemExit(f"make_golden.py needs a checkout of the reference: {ref} has no interact_drive/")
     sys.path.insert(0, str(REPO / "oracle" / "tf_shim"))
-    sys.path.insert(0, str(REF))
-    os.chdir(REF)  # the library imports the `experiments` package relative to the repo root
+    sys.path.insert(0, str(ref))
+    os.chdir(ref)  # the library imports the `experiments` package relative to the repo root
 
 
 def _f(x):
@@ -341,8 +340,8 @@ SIMPLE = {"primitives": part_primitives, "features": part_features, "mpc_reward"
           "plans": part_plans, "planner_kats": part_planner_kats}
 
 
-def run_part(part: str, outdir: Path = HERE):
-    _setup_reference_imports()
+def run_part(part: str, ref: Path, outdir: Path = HERE):
+    _setup_reference_imports(ref)
     t0 = time.time()
     if part in SIMPLE:
         data = SIMPLE[part]()
@@ -363,10 +362,15 @@ def main():
     ap.add_argument("--all", action="store_true")
     ap.add_argument("--jobs", type=int, default=8)
     ap.add_argument("--outdir", default=str(HERE), help="where to write the JSON (default: tests/golden)")
+    ap.add_argument("--reference", default=os.environ.get("L4DC_REFERENCE_DIR"),
+                    help="checkout of the reference (default: $L4DC_REFERENCE_DIR)")
     args = ap.parse_args()
+    if not args.reference:
+        ap.error("--reference DIR (or L4DC_REFERENCE_DIR) must name a checkout of the reference")
+    ref = Path(args.reference).resolve()
     parts = list(SIMPLE) + ["episode:%s:%s:%s" % e for e in EPISODES]
     if args.part:
-        run_part(args.part, Path(args.outdir).resolve())
+        run_part(args.part, ref, Path(args.outdir).resolve())
         return
     if not args.all:
         ap.error("--part NAME or --all")
@@ -374,7 +378,7 @@ def main():
     while pending or running:
         while pending and len(running) < args.jobs:
             p = pending.pop(0)
-            running.append((p, subprocess.Popen([sys.executable, __file__, "--part", p])))
+            running.append((p, subprocess.Popen([sys.executable, __file__, "--part", p, "--reference", str(ref)])))
         time.sleep(2)
         for item in list(running):
             if item[1].poll() is not None:
