@@ -184,6 +184,27 @@ int ocd_solve_batch(const ocd_params *p, const float *world /*[C][4][B]*/,
                     float *plan, float *losses, int32_t *best, float *all_plans,
                     int64_t B, void *stream);
 
+/* Vector-Jacobian product of ocd_solve_batch's plan with respect to the weights and the initial world: given
+ * plan_bar = d loss / d plan, weights_bar[k][b] = d loss / d w_k of problem b's weight vector and world_bar = d loss /
+ * d world, for the fixed-budget SGD plan (optimizer == 0; L-BFGS's line search is not differentiable: OCD_EUNSUP).
+ * The derivative follows the start ocd_solve_batch picked (best, its output) through the n_iter SGD steps
+ * (naive_planner.py:151-153) and through the start itself (the extra-init starts depend on the robot's speed when
+ * cur_speed is NULL); the argmin over starts, clip masks and min / max selections have zero derivative almost
+ * everywhere.  The other cars enter world_bar through the planner's prediction of them (naive_planner.py:53-66).
+ * Nothing is summed across problems: with a shared or indexed weight table the caller adds the rows of weights_bar
+ * that use the same vector.  Inputs as for ocd_solve_batch (the same params, world, weights, other controls and
+ * cur_speed); world_bar may be NULL.  workspace: device memory of at least ocd_solve_vjp_workspace_bytes() bytes
+ * (n_iter * H * 2 * B floats: the recomputed iterates); too small -> OCD_EINVAL.
+ * Outputs: weights_bar [K][B], world_bar [C][4][B] or NULL. */
+int ocd_solve_vjp_workspace_bytes(const ocd_params *p, int64_t B, size_t *bytes);
+int ocd_solve_vjp_batch(const ocd_params *p, const float *world /*[C][4][B]*/,
+                        const float *other_controls, int64_t Bo,
+                        const float *weights, int64_t Bw, const int32_t *weight_idx,
+                        const float *cur_speed,
+                        const int32_t *best /*[B], from ocd_solve_batch*/, const float *plan_bar /*[H][2][B]*/,
+                        float *weights_bar /*[K][B]*/, float *world_bar /*[C][4][B] or NULL*/,
+                        void *workspace, size_t workspace_bytes, int64_t B, void *stream);
+
 /* The receding-horizon episode of MPC_ORD.eval_weights_for_init
  * (interact_drive/reward_design/mpc_ord.py:87-103): T times CarWorld.step
  * (interact_drive/world.py:79-109; ReplanningCarWorld.step experiments/replanning_world.py:29-36),

@@ -70,6 +70,8 @@ _PROTOTYPES = {
     "ocd_feature_jacobian_batch": (C.c_int, [_P, _P, _P, _P, _I64, _P, _P, _I64, _P]),
     "ocd_feature_hessian_batch": (C.c_int, [_P, _P, _P, _P, _I64, _P, _I64, _P]),
     "ocd_solve_batch": (C.c_int, [_P, _P, _P, _I64, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _P]),
+    "ocd_solve_vjp_workspace_bytes": (C.c_int, [_P, _I64, C.POINTER(C.c_size_t)]),
+    "ocd_solve_vjp_batch": (C.c_int, [_P, _P, _P, _I64, _P, _I64, _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _I64, _P]),
     "ocd_episode_batch": (C.c_int, [_P, _P, _P, _P, _P, _I64, _P, _P, _P, _I32, _I32,
                                     _P, _P, _P, _P, _P, _I64, _P]),
     "ocd_ctx_create": (C.c_int, [C.c_int, C.POINTER(_P)]),

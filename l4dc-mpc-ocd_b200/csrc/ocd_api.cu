@@ -19,6 +19,7 @@
 
 #include "ocd_kernels.cuh"
 #include "ocd_hessian.cuh"
+#include "ocd_vjp.cuh"
 
 namespace ocd {
 
@@ -29,7 +30,9 @@ namespace ocd {
     extern template int launch_episode_t<HT, NO, LT, false>(const KParams &, const ocd_scenario &,           \
                                                             const EpisodeArgs &, cudaStream_t);              \
     extern template int launch_episode_t<HT, NO, LT, true>(const KParams &, const ocd_scenario &,            \
-                                                           const EpisodeArgs &, cudaStream_t);
+                                                           const EpisodeArgs &, cudaStream_t);               \
+    extern template int launch_solve_vjp_t<HT, NO, LT, false>(const KParams &, const VjpArgs &, cudaStream_t); \
+    extern template int launch_solve_vjp_t<HT, NO, LT, true>(const KParams &, const VjpArgs &, cudaStream_t);
 OCD_EXTERN(5, 1, 3)   // finite_horizon, local_opt, the bench shape
 OCD_EXTERN(5, 2, 2)   // replanning
 OCD_EXTERN(6, 1, 3)   // finite_horizon validation (H=6, n_iter=200)
@@ -39,8 +42,9 @@ OCD_EXTERN(0, 0, 3)   // any horizon / cars on three lanes: segmented adjoint
 OCD_EXTERN(0, 0, 0)   // any other shape: runtime H, cars, lanes (segmented adjoint)
 #undef OCD_EXTERN
 // FAST k_solve alone, compile-time car count: the 3..6-car points of the synthetic sweep
-#define OCD_EXTERN_SOLVE(HT, NO, LT) \
-    extern template int launch_solve_t<HT, NO, LT, false>(const KParams &, const SolveArgs &, cudaStream_t);
+#define OCD_EXTERN_SOLVE(HT, NO, LT)                                                                       \
+    extern template int launch_solve_t<HT, NO, LT, false>(const KParams &, const SolveArgs &, cudaStream_t); \
+    extern template int launch_solve_vjp_t<HT, NO, LT, false>(const KParams &, const VjpArgs &, cudaStream_t);
 OCD_EXTERN_SOLVE(5, 2, 3)
 OCD_EXTERN_SOLVE(5, 3, 3)
 OCD_EXTERN_SOLVE(5, 4, 3)
@@ -488,6 +492,21 @@ static int launch_solve(const KParams &k, bool precise, const SolveArgs &a, cuda
     OCD_DISPATCH(launch_solve_t, false, k, a, st);
 }
 
+// the solve's own dispatch: the reverse pass re-runs the iterations of the specialisation the forward ran
+static int launch_solve_vjp(const KParams &k, bool precise, const VjpArgs &a, cudaStream_t st) {
+    if (precise) OCD_DISPATCH(launch_solve_vjp_t, true, k, a, st);
+    if (k.L == 3 && k.NO >= 1 && k.NO <= 5 && !((k.H == 15 || k.H == 50) && runtime_h_forced())) {
+        switch (k.NO) {
+            case 1: OCD_SOLVE_SWITCH(launch_solve_vjp_t, 1, k, a, st); break;
+            case 2: OCD_SOLVE_SWITCH(launch_solve_vjp_t, 2, k, a, st); break;
+            case 3: OCD_SOLVE_SWITCH(launch_solve_vjp_t, 3, k, a, st); break;
+            case 4: OCD_SOLVE_SWITCH(launch_solve_vjp_t, 4, k, a, st); break;
+            default: OCD_SOLVE_SWITCH(launch_solve_vjp_t, 5, k, a, st); break;
+        }
+    }
+    OCD_DISPATCH(launch_solve_vjp_t, false, k, a, st);
+}
+
 static int launch_episode(const KParams &k, bool precise, const ocd_scenario &sc, const EpisodeArgs &a,
                           cudaStream_t st) {
     if (precise) OCD_DISPATCH(launch_episode_t, true, k, sc, a, st);
@@ -676,6 +695,39 @@ int ocd_solve_batch(const ocd_params *p, const float *world, const float *other_
         return cuda_status();
     }
     return launch_solve(k, p->math_mode == 1, a, (cudaStream_t)stream);
+}
+
+static size_t vjp_workspace_bytes(const KParams &k, int64_t B) {
+    return (size_t)k.n_iter * (size_t)k.H * 2 * (size_t)B * sizeof(float);
+}
+
+int ocd_solve_vjp_workspace_bytes(const ocd_params *p, int64_t B, size_t *bytes) {
+    KParams k;
+    const int rc = digest(p, k);
+    if (rc) return rc;
+    if (!bytes || B < 0) return OCD_EINVAL;
+    if (k.optimizer != 0) return OCD_EUNSUP;      // L-BFGS: its line search is not differentiable
+    *bytes = vjp_workspace_bytes(k, B);
+    return OCD_OK;
+}
+
+int ocd_solve_vjp_batch(const ocd_params *p, const float *world, const float *other_controls, int64_t Bo,
+                        const float *weights, int64_t Bw, const int32_t *weight_idx, const float *cur_speed,
+                        const int32_t *best, const float *plan_bar, float *weights_bar, float *world_bar,
+                        void *workspace, size_t workspace_bytes, int64_t B, void *stream) {
+    KParams k;
+    int rc = digest(p, k);
+    if (rc) return rc;
+    if (k.optimizer != 0) return OCD_EUNSUP;
+    if (B == 0) return OCD_OK;
+    if (!world || !best || !plan_bar || !weights_bar || B < 0) return OCD_EINVAL;
+    if ((rc = check_weights(weights, Bw, weight_idx, B))) return rc;
+    if (k.other_mode == 1 && (!other_controls || (Bo != 1 && Bo != B))) return OCD_EINVAL;
+    const size_t need = vjp_workspace_bytes(k, B);
+    if (workspace_bytes < need || (need > 0 && !workspace)) return OCD_EINVAL;
+    VjpArgs a{world, other_controls, Bo, weights, Bw, weight_idx, cur_speed, best, plan_bar, weights_bar, world_bar,
+              static_cast<float *>(workspace), B};
+    return launch_solve_vjp(k, p->math_mode == 1, a, (cudaStream_t)stream);
 }
 
 int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc, const float *robot_init,

@@ -71,6 +71,7 @@ __device__ __forceinline__ HD hd_bump(HD z, float c, float hw) {
     return hd_const(0.0f);
 }
 
+#ifndef OCD_HD_ONLY   // translation units that only use the hyper-dual arithmetic (ocd_vjp.cuh in ocd_inst.cu)
 // One thread: problem b, control pair (i, j) with i <= j (flat indices into [H][2]).  hess [K][2H][2H][B].
 __global__ void __launch_bounds__(128)
 k_feature_hessian(const __grid_constant__ KParams k, const float *world, const float *controls,
@@ -151,5 +152,6 @@ k_feature_hessian(const __grid_constant__ KParams k, const float *world, const f
             hess[((size_t)(q * n + j) * n + i) * B + b] = phi_sum[q].ab;
         }
 }
+#endif
 
 }  // namespace ocd

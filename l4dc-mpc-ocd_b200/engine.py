@@ -229,6 +229,41 @@ class Engine:
         self._kernel_launches += 1 if B else 0
         return out
 
+    def solve_vjp_soa(self, p: PlannerParams, world, weights, Bw: int, best, plan_bar, weight_idx=None,
+                      other_controls=None, Bo: int = 0, cur_speed=None, world_bar: bool = True):
+        """Vector-Jacobian product of solve_soa's plan (``ocd_solve_vjp_batch``): the same inputs, solve_soa's `best`
+        and plan_bar [H][2][B] = d loss / d plan -> dict(weights_bar [K][B]: d loss / d (problem b's weight vector),
+        world_bar [C][4][B] (with world_bar=True)).  Rows are per problem; problems sharing a weight vector are not
+        summed here.  The workspace (n_iter * H * 2 * B floats) is allocated on the device for the call."""
+        B = world.shape[-1]
+        dev = self.device
+        f32, i32 = torch.float32, torch.int32
+        _check_soa("world", world, f32, dev, (p.C, 4, B))
+        _check_soa("weights", weights, f32, dev, (p.K, Bw))
+        _check_soa("weight_idx", weight_idx, i32, dev, (B,))
+        _check_soa("cur_speed", cur_speed, f32, dev, (B,))
+        _check_soa("best", best, i32, dev, (B,))
+        _check_soa("plan_bar", plan_bar, f32, dev, (p.H, 2, B))
+        if p.other_mode == 1:
+            if other_controls is None or Bo not in (1, B):
+                raise ValueError("other_mode=1 needs other_controls [C-1][H][2][Bo] with Bo in (1, B)")
+            _check_soa("other_controls", other_controls, f32, dev, (p.C - 1, p.H, 2, Bo))
+        ps = p.c_struct()
+        nbytes = C.c_size_t(0)
+        N.check(N.lib.ocd_solve_vjp_workspace_bytes(C.addressof(ps), B, C.byref(nbytes)), "ocd_solve_vjp_workspace_bytes")
+        ws = torch.empty((nbytes.value // 4,), dtype=f32, device=dev)
+        out = dict(weights_bar=torch.empty((p.K, B), dtype=f32, device=dev))
+        if world_bar:
+            out["world_bar"] = torch.empty((p.C, 4, B), dtype=f32, device=dev)
+        with torch.cuda.device(dev):
+            rc = N.lib.ocd_solve_vjp_batch(C.addressof(ps), _ptr(world), _ptr(other_controls), Bo, _ptr(weights), Bw,
+                                           _ptr(weight_idx), _ptr(cur_speed), _ptr(best), _ptr(plan_bar),
+                                           _ptr(out["weights_bar"]), _ptr(out.get("world_bar")), _ptr(ws),
+                                           nbytes.value, B, self._stream())
+        N.check(rc, "ocd_solve_vjp_batch")
+        self._kernel_launches += 1 if B else 0
+        return out
+
     def episodes_soa(self, p: PlannerParams, sc: Scenario, robot_init, plan_weights, Bw: int, true_weights, T: int,
                      weight_idx=None, other_init=None, unlucky_idx=None, t0: int = 0, trace: bool = False,
                      final_world: bool = False, out=None):

@@ -1,6 +1,7 @@
 """The two planner entry points as PyTorch custom ops (``torch.ops.ocd_b200.solve`` /
-``torch.ops.ocd_b200.episodes``): device tensors in, device tensors out, launched on the current stream
-through the same C ABI as everything else.  Registering them makes the engine usable from code that
+``torch.ops.ocd_b200.episodes``) and the reverse pass of the solve (``torch.ops.ocd_b200.solve_vjp``, which is
+also ``solve``'s autograd formula: gradients of the plan reach ``world`` and ``weights``): device tensors in,
+device tensors out, launched on the current stream through the same C ABI as everything else.  Registering them makes the engine usable from code that
 composes torch ops (and gives them fake-tensor shape functions); there is deliberately no CPU kernel --
 calling them with CPU tensors is an error, not a fallback.
 
@@ -59,6 +60,63 @@ def _(world, weights, weight_idx, other_controls, params):
     p = unpack_params(params)
     B = world.shape[-1]
     return (world.new_empty((p.H, 2, B)), world.new_empty((p.S, B)), world.new_empty((B,), dtype=torch.int32))
+
+
+@torch.library.custom_op("ocd_b200::solve_vjp", mutates_args=())
+def solve_vjp(world: torch.Tensor, weights: torch.Tensor, weight_idx: Optional[torch.Tensor],
+              other_controls: Optional[torch.Tensor], best: torch.Tensor, plan_bar: torch.Tensor,
+              params: List[float]) -> Tuple[torch.Tensor, torch.Tensor]:
+    """solve's inputs, its `best` [B] i32 and plan_bar [H,2,B] = d loss / d plan -> (weights_bar [K,B]: per problem,
+    d loss / d the weight vector problem b planned with; world_bar [C,4,B])."""
+    p = unpack_params(params)
+    eng = _engine(world)
+    Bo = 0 if other_controls is None else other_controls.shape[-1]
+    out = eng.solve_vjp_soa(p, world.contiguous(), weights.contiguous(), weights.shape[-1], best.contiguous(),
+                            plan_bar.contiguous(), None if weight_idx is None else weight_idx.contiguous(),
+                            None if other_controls is None else other_controls.contiguous(), Bo)
+    return out["weights_bar"], out["world_bar"]
+
+
+@solve_vjp.register_fake
+def _(world, weights, weight_idx, other_controls, best, plan_bar, params):
+    p = unpack_params(params)
+    B = world.shape[-1]
+    return world.new_empty((p.K, B)), world.new_empty((p.C, 4, B))
+
+
+def _solve_setup_context(ctx, inputs, output):
+    world, weights, weight_idx, other_controls, params = inputs
+    ctx.set_materialize_grads(False)          # an output nobody differentiates arrives as None, not as zeros
+    ctx.save_for_backward(world, weights, weight_idx, other_controls, output[2])
+    ctx.params = params
+
+
+def _solve_backward(ctx, plan_bar, losses_bar, best_bar):
+    if losses_bar is not None:
+        raise RuntimeError("ocd_b200::solve: the losses are not differentiable (only the plan is: the gradient follows "
+                           "the winning start through the SGD iterations); detach them before using them in a loss")
+    if ctx.needs_input_grad[3]:
+        raise RuntimeError("ocd_b200::solve: gradients with respect to other_controls are not supported; "
+                           "pass other_controls without requires_grad")
+    world, weights, weight_idx, other_controls, best = ctx.saved_tensors
+    if plan_bar is None:
+        return None, None, None, None, None
+    weights_bar, world_bar = torch.ops.ocd_b200.solve_vjp(world, weights, weight_idx, other_controls, best,
+                                                          plan_bar.contiguous(), ctx.params)
+    Bw, B = weights.shape[-1], world.shape[-1]
+    if weight_idx is not None:
+        # rows of the problems that share a vector, summed deterministically: index_put_ with accumulate=True sorts by
+        # index on CUDA (index_add_ would add with float atomics, in an order that changes from run to run)
+        wb = torch.zeros((Bw, weights_bar.shape[0]), dtype=weights_bar.dtype, device=weights_bar.device)
+        wb.index_put_((weight_idx.long(),), weights_bar.t(), accumulate=True)
+        weights_bar = wb.t()
+    elif Bw == 1 and B != 1:
+        weights_bar = weights_bar.sum(dim=1, keepdim=True)
+    return (world_bar if ctx.needs_input_grad[0] else None, weights_bar if ctx.needs_input_grad[1] else None,
+            None, None, None)
+
+
+solve.register_autograd(_solve_backward, setup_context=_solve_setup_context)
 
 
 @torch.library.custom_op("ocd_b200::episodes", mutates_args=())
