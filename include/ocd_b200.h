@@ -231,6 +231,29 @@ int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc,
                       float *traj_states, float *final_world,
                       int64_t B, void *stream);
 
+/* Vector-Jacobian product of ocd_episode_batch's returns: given returns_bar = d loss / d returns,
+ *   plan_weights_bar [K][B]         d loss / d (world b's planning weight vector)
+ *   robot_init_bar   [4][B] or NULL d loss / d robot_init
+ *   true_weights_bar [K][B] or NULL d loss / d true_weights, per world (returns_bar[b] * sum_t features(past state))
+ * for the fixed-budget SGD planner (optimizer == 1: OCD_EUNSUP).  The derivative follows the episode's own
+ * trajectory: traj_states [T][C][4][B], traj_best [T][B] and traj_controls [T][2][B] are what ocd_episode_batch
+ * wrote for the same params, scenario, weights and T.  Every step contributes the Jacobian of its applied control with
+ * respect to the weights and the robot's state (the solve VJP of the winning start, seeded on plan[0]) and the
+ * simulator step's; the scripted cars depend on neither, and the argmin over starts, clip masks and min / max
+ * selections are not differentiated.  Nothing is summed across worlds.  workspace: device memory of at least
+ * min_bytes from ocd_episode_vjp_workspace_bytes (the Jacobian rows and the iterates of one step); full_bytes holds
+ * the iterates of all T steps at once, so fewer launches; anything in between is used as far as it goes, with the
+ * same results.  Too small -> OCD_EINVAL.  T == 0 writes zeros. */
+int ocd_episode_vjp_workspace_bytes(const ocd_params *p, int32_t T, int64_t B, size_t *min_bytes, size_t *full_bytes);
+int ocd_episode_vjp_batch(const ocd_params *p, const ocd_scenario *sc,
+                          const float *plan_weights, int64_t Bw, const int32_t *weight_idx,
+                          const float *true_weights, int32_t T,
+                          const float *traj_states /*[T][C][4][B]*/, const int32_t *traj_best /*[T][B]*/,
+                          const float *traj_controls /*[T][2][B]*/, const float *returns_bar /*[B]*/,
+                          float *plan_weights_bar /*[K][B]*/, float *robot_init_bar /*[4][B] or NULL*/,
+                          float *true_weights_bar /*[K][B] or NULL*/,
+                          void *workspace, size_t workspace_bytes, int64_t B, void *stream);
+
 /* ---- host-buffer convenience layer (what a Python/ctypes caller without torch uses) ---------
  * An ocd_ctx owns a device, a stream, pinned staging buffers and device buffers that grow on
  * demand.  The *_host calls take HOST pointers with the same layouts as above, copy in, run the

@@ -74,6 +74,9 @@ _PROTOTYPES = {
     "ocd_solve_vjp_batch": (C.c_int, [_P, _P, _P, _I64, _P, _I64, _P, _P, _P, _P, _P, _P, _P, C.c_size_t, _I64, _P]),
     "ocd_episode_batch": (C.c_int, [_P, _P, _P, _P, _P, _I64, _P, _P, _P, _I32, _I32,
                                     _P, _P, _P, _P, _P, _I64, _P]),
+    "ocd_episode_vjp_workspace_bytes": (C.c_int, [_P, _I32, _I64, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
+    "ocd_episode_vjp_batch": (C.c_int, [_P, _P, _P, _I64, _P, _P, _I32, _P, _P, _P, _P, _P, _P, _P, _P, C.c_size_t,
+                                        _I64, _P]),
     "ocd_ctx_create": (C.c_int, [C.c_int, C.POINTER(_P)]),
     "ocd_ctx_destroy": (None, [_P]),
     "ocd_host_register": (C.c_int, [_P, C.c_size_t]),

@@ -32,7 +32,11 @@ namespace ocd {
     extern template int launch_episode_t<HT, NO, LT, true>(const KParams &, const ocd_scenario &,            \
                                                            const EpisodeArgs &, cudaStream_t);               \
     extern template int launch_solve_vjp_t<HT, NO, LT, false>(const KParams &, const VjpArgs &, cudaStream_t); \
-    extern template int launch_solve_vjp_t<HT, NO, LT, true>(const KParams &, const VjpArgs &, cudaStream_t);
+    extern template int launch_solve_vjp_t<HT, NO, LT, true>(const KParams &, const VjpArgs &, cudaStream_t);    \
+    extern template int launch_episode_jac_t<HT, NO, LT, false>(const KParams &, const ocd_scenario &,         \
+                                                                const EpisodeVjpArgs &, int, cudaStream_t);  \
+    extern template int launch_episode_jac_t<HT, NO, LT, true>(const KParams &, const ocd_scenario &,          \
+                                                               const EpisodeVjpArgs &, int, cudaStream_t);
 OCD_EXTERN(5, 1, 3)   // finite_horizon, local_opt, the bench shape
 OCD_EXTERN(5, 2, 2)   // replanning
 OCD_EXTERN(6, 1, 3)   // finite_horizon validation (H=6, n_iter=200)
@@ -513,6 +517,13 @@ static int launch_episode(const KParams &k, bool precise, const ocd_scenario &sc
     OCD_DISPATCH(launch_episode_t, false, k, sc, a, st);
 }
 
+// the episode's own dispatch: the reverse pass re-runs the iterations of the specialisation k_episode ran
+static int launch_episode_jac(const KParams &k, bool precise, const ocd_scenario &sc, const EpisodeVjpArgs &a,
+                              int group, cudaStream_t st) {
+    if (precise) OCD_DISPATCH(launch_episode_jac_t, true, k, sc, a, group, st);
+    OCD_DISPATCH(launch_episode_jac_t, false, k, sc, a, group, st);
+}
+
 // the same two dispatches, asking which kernel form would run (ocd_kernel_form)
 static int form_of(const KParams &k, bool precise, long long B, bool episode) {
     if (precise) OCD_DISPATCH(form_t, true, k, B, episode);
@@ -750,6 +761,62 @@ int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc, const float *
     EpisodeArgs a{robot_init, other_init, plan_weights, Bw, weight_idx, true_weights, unlucky_idx, t0, T,
                   returns, traj_controls, traj_best, traj_states, final_world, B, pick_P(B)};
     return launch_episode(k, p->math_mode == 1, *sc, a, (cudaStream_t)stream);
+}
+
+// workspace of ocd_episode_vjp_batch: the Jacobian rows [T][2][K + 4][B], then the iterates of the steps in flight,
+// [N + 1][H][2][B] per step
+static size_t episode_jac_bytes(const KParams &k, int32_t T, int64_t B) {
+    return (size_t)T * 2 * (size_t)(k.K + 4) * (size_t)B * sizeof(float);
+}
+static size_t episode_step_bytes(const KParams &k, int64_t B) {
+    return (size_t)(k.n_iter + 1) * (size_t)k.H * 2 * (size_t)B * sizeof(float);
+}
+
+int ocd_episode_vjp_workspace_bytes(const ocd_params *p, int32_t T, int64_t B, size_t *min_bytes, size_t *full_bytes) {
+    KParams k;
+    const int rc = digest(p, k);
+    if (rc) return rc;
+    if (!min_bytes || !full_bytes || B < 0 || T < 0) return OCD_EINVAL;
+    if (k.optimizer != 0) return OCD_EUNSUP;      // L-BFGS: its line search is not differentiable
+    const size_t jac = episode_jac_bytes(k, T, B), step = episode_step_bytes(k, B);
+    *min_bytes = jac + (T > 0 ? step : 0);
+    *full_bytes = jac + (size_t)T * step;
+    return OCD_OK;
+}
+
+int ocd_episode_vjp_batch(const ocd_params *p, const ocd_scenario *sc, const float *plan_weights, int64_t Bw,
+                          const int32_t *weight_idx, const float *true_weights, int32_t T, const float *traj_states,
+                          const int32_t *traj_best, const float *traj_controls, const float *returns_bar,
+                          float *plan_weights_bar, float *robot_init_bar, float *true_weights_bar, void *workspace,
+                          size_t workspace_bytes, int64_t B, void *stream) {
+    KParams k;
+    int rc = digest(p, k);
+    if (rc) return rc;
+    if (k.optimizer != 0) return OCD_EUNSUP;
+    if (B == 0) return OCD_OK;
+    if (!sc || !true_weights || !returns_bar || !plan_weights_bar || B < 0 || T < 0) return OCD_EINVAL;
+    if (T > 0 && (!traj_states || !traj_best || !traj_controls)) return OCD_EINVAL;
+    if (sc->n_other != k.NO) return OCD_EINVAL;
+    for (int j = 0; j < k.NO; ++j)
+        if (sc->plan_len[j] < 0 || sc->plan_len[j] > OCD_MAX_PLAN || (sc->kind[j] != 0 && sc->kind[j] != 1))
+            return OCD_EINVAL;
+    if ((rc = check_weights(plan_weights, Bw, weight_idx, B))) return rc;
+    const size_t jac = episode_jac_bytes(k, T, B), step = episode_step_bytes(k, B);
+    const size_t need = jac + (T > 0 ? step : 0);
+    if (workspace_bytes < need || (need > 0 && !workspace)) return OCD_EINVAL;
+    EpisodeVjpArgs a{plan_weights, Bw, weight_idx, true_weights, T, 0, traj_states, traj_best, traj_controls,
+                     returns_bar, plan_weights_bar, robot_init_bar, true_weights_bar, static_cast<float *>(workspace),
+                     reinterpret_cast<float *>(static_cast<char *>(workspace) + jac), B};
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (T > 0) {
+        // as many steps in flight as the workspace holds (at most 65 535: gridDim.y)
+        size_t group = (workspace_bytes - jac) / step;
+        if (group > (size_t)T) group = (size_t)T;
+        if (group > 65535) group = 65535;
+        if ((rc = launch_episode_jac(k, p->math_mode == 1, *sc, a, (int)group, st))) return rc;
+    }
+    k_episode_adjoint<<<(unsigned)((B + kVjpThreads - 1) / kVjpThreads), kVjpThreads, 0, st>>>(k, a);
+    return cuda_status();
 }
 
 // ---- host-buffer layer ------------------------------------------------------------------------

@@ -1,4 +1,5 @@
-// ocd_inst.cu -- one (H, other cars, lanes, math mode) specialisation of k_solve / k_episode / k_solve_vjp.
+// ocd_inst.cu -- one (H, other cars, lanes, math mode) specialisation of k_solve / k_episode / k_solve_vjp /
+// k_episode_jac.
 // Compiled once per combination by the Makefile:
 //   nvcc -DOCD_HT=5 -DOCD_NO=1 -DOCD_LT=3 -DOCD_PRECISE=0 -c ocd_inst.cu -o build/inst_5_1_3_0.o
 //   (+ -DOCD_SOLVE_ONLY for build/solve_<HT>_<NO>_<LT>.o: FAST k_solve alone)
@@ -16,6 +17,9 @@ template int launch_solve_vjp_t<OCD_HT, OCD_NO, OCD_LT, (OCD_PRECISE != 0)>(cons
 #ifndef OCD_SOLVE_ONLY   // the many-car sweep specialisations build k_solve only
 template int launch_episode_t<OCD_HT, OCD_NO, OCD_LT, (OCD_PRECISE != 0)>(const KParams &, const ocd_scenario &,
                                                                   const EpisodeArgs &, cudaStream_t);
+// the episode's reverse pass re-runs the iterations of the episode's specialisation (not the solve's)
+template int launch_episode_jac_t<OCD_HT, OCD_NO, OCD_LT, (OCD_PRECISE != 0)>(const KParams &, const ocd_scenario &,
+                                                                      const EpisodeVjpArgs &, int, cudaStream_t);
 #endif
 }  // namespace ocd
 

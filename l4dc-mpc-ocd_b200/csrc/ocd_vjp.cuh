@@ -26,6 +26,10 @@
 // (thread b touches element b).  The reverse pass then reads them back in reverse order; it runs in precise arithmetic
 // (libdevice sin / cos / exp, IEEE division) whatever the math mode, like the Hessian and L-BFGS kernels.  Outputs are
 // per problem, weights_bar [K][B] and world_bar [C][4][B]: no reduction across problems, no atomics.
+//
+// The second half of the file is the reverse pass through whole episodes (ocd_episode_vjp_batch): the same recompute
+// phase and reverse sweep per (world, step), seeded on the applied control, then the robot's adjoint along the episode
+// (see k_episode_vjp below).
 #pragma once
 
 #include "ocd_kernels.cuh"
@@ -200,39 +204,84 @@ __device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, 
     s0bar[3] = fmaf(k.lr, lthd, s0bar[3]);
 }
 
-// The reverse pass of problem b (start s, iterates already in the workspace); writes weights_bar and world_bar.
-static __device__ __noinline__ void vjp_reverse(const KParams &k, const VjpArgs &a, long long b, int s) {
-    const long long B = a.B;
-    const int H = k.H, NO = k.NO;
-    float oth[OCD_MAX_H * OCD_MAX_OTHER * 2], obar[OCD_MAX_H * OCD_MAX_OTHER * 2];
-    for (int j = 0; j < NO; ++j) {
-        const float *st = a.world + (size_t)(j + 1) * 4 * B + b;
-        const float *oc = nullptr;
-        long long ocs = 0;
-        if (k.other_mode == 1) {
-            ocs = a.Bo;
-            oc = a.other_controls + (size_t)j * H * 2 * a.Bo + (a.Bo == 1 ? 0 : b);
+// Where the planner's model of the other cars takes its known controls from (other_mode == 1): a solve's
+// other_controls [NO][H][2][Bo], or an episode's scenario -- k_episode's model, written out per car into buf [H][2]:
+// a fixed-plan car's plan replayed from index 0 and then its control (quirk Q4), zero for every other car.
+struct OtherControls {
+    const float *table;            // [NO][H][2][Bo] or null
+    long long    Bo;
+    const ocd_scenario *sc;        // episodes (table null)
+    __device__ __forceinline__ const float *car(const KParams &k, int j, long long b, float *buf, long long &ocs) const {
+        ocs = 0;
+        if (k.other_mode != 1) return nullptr;
+        if (sc) {
+            for (int t = 0; t < k.H; ++t) {
+                float oa = 0.0f, oo = 0.0f;
+                if (sc->kind[j] == 1) {
+                    const bool in_plan = t < sc->plan_len[j];
+                    oa = in_plan ? sc->plan[j][t][0] : sc->control[j][0];
+                    oo = in_plan ? sc->plan[j][t][1] : sc->control[j][1];
+                }
+                buf[2 * t] = oa;
+                buf[2 * t + 1] = oo;
+            }
+            ocs = 1;
+            return buf;
         }
+        ocs = Bo;
+        return table + (size_t)j * k.H * 2 * Bo + (Bo == 1 ? 0 : b);
+    }
+};
+
+// The other cars' predicted positions [H][NO][2] in precise arithmetic (the reverse pass's own copy of the slab).
+__device__ __forceinline__ void vjp_predict_others(const KParams &k, const float *world, long long B, long long b,
+                                                   const OtherControls &ocs_src, float *oth) {
+    float buf[2 * OCD_MAX_H];
+    for (int j = 0; j < k.NO; ++j) {
+        const float *st = world + (size_t)(j + 1) * 4 * B + b;
+        long long ocs;
+        const float *oc = ocs_src.car(k, j, b, buf, ocs);
         predict_other<true>(k, st[0], st[B], st[2 * B], st[3 * B], oc, ocs, oth, j, 1);
     }
-    for (int i = 0; i < H * NO * 2; ++i) obar[i] = 0.0f;
-    const float s0[4] = {a.world[b], a.world[B + b], a.world[2 * B + b], a.world[3 * B + b]};
-    const float *w = a.weights + weight_column(a.weight_idx, a.Bw, b);
-    const int ws = (int)a.Bw;
-    float u[2 * OCD_MAX_H], ubar[2 * OCD_MAX_H], wbar[kVjpK], s0bar[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-    for (int i = 0; i < 2 * H; ++i) ubar[i] = a.plan_bar[(size_t)i * B + b];
-#pragma unroll
-    for (int q = 0; q < kVjpK; ++q) wbar[q] = 0.0f;
+}
+
+// The reverse pass over the stored iterates of one problem (it: u^0 .. u^{N-1} at element stride B, offset to the
+// problem).  On entry ubar holds plan_bar and wbar [K], s0bar [4], obar [H][NO][2] are zero; on exit wbar and s0bar
+// hold the VJP with respect to the weights and the robot's initial state -- the extra-init starts' dependence on the
+// speed included when the start was built from v0 -- and obar that with respect to the predicted positions.
+__device__ __forceinline__ void vjp_sweep(const KParams &k, const float *w, int ws, const float (&s0)[4],
+                                          const float *oth, const float *it, long long B, int s, bool speed_is_v0,
+                                          float *ubar, float *wbar, float *s0bar, float *obar) {
+    const int H = k.H;
+    float u[2 * OCD_MAX_H];
     for (int n = k.n_iter - 1; n >= 0; --n) {
-        for (int i = 0; i < 2 * H; ++i) u[i] = a.iters[((size_t)n * 2 * H + i) * B + b];
+        for (int i = 0; i < 2 * H; ++i) u[i] = it[((size_t)n * 2 * H + i) * B];
         vjp_iteration(k, w, ws, s0, oth, u, ubar, wbar, s0bar, obar);
     }
     // the start: a0 = friction * cur_speed^2 for the extra-init starts (naive_planner.py:114-116), cur_speed = v0
-    if (s >= 3 && !a.cur_speed) {
+    if (s >= 3 && speed_is_v0) {
         float sa = 0.0f;
         for (int t = 0; t < H; ++t) sa += ubar[2 * t];
         s0bar[2] = fmaf(sa, 2.0f * k.mu * s0[2], s0bar[2]);
     }
+}
+
+// The reverse pass of problem b (start s, iterates already in the workspace); writes weights_bar and world_bar.
+static __device__ __noinline__ void vjp_reverse(const KParams &k, const VjpArgs &a, long long b, int s) {
+    const long long B = a.B;
+    const int H = k.H, NO = k.NO;
+    const OtherControls ocs_src{a.other_controls, a.Bo, nullptr};
+    float oth[OCD_MAX_H * OCD_MAX_OTHER * 2], obar[OCD_MAX_H * OCD_MAX_OTHER * 2];
+    vjp_predict_others(k, a.world, B, b, ocs_src, oth);
+    for (int i = 0; i < H * NO * 2; ++i) obar[i] = 0.0f;
+    const float s0[4] = {a.world[b], a.world[B + b], a.world[2 * B + b], a.world[3 * B + b]};
+    const float *w = a.weights + weight_column(a.weight_idx, a.Bw, b);
+    const int ws = (int)a.Bw;
+    float ubar[2 * OCD_MAX_H], wbar[kVjpK], s0bar[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+    for (int i = 0; i < 2 * H; ++i) ubar[i] = a.plan_bar[(size_t)i * B + b];
+#pragma unroll
+    for (int q = 0; q < kVjpK; ++q) wbar[q] = 0.0f;
+    vjp_sweep(k, w, ws, s0, oth, a.iters + b, B, s, !a.cur_speed, ubar, wbar, s0bar, obar);
 #pragma unroll
     for (int q = 0; q < kVjpK; ++q)
         if (q < k.K) a.weights_bar[(size_t)q * B + b] = wbar[q];
@@ -271,37 +320,33 @@ static __device__ __noinline__ void vjp_reverse(const KParams &k, const VjpArgs 
     }
 }
 
-// Phase 1 re-runs the winning start with the iteration code k_solve runs for this specialisation (HT, NOT_, LT,
-// PRECISE): the register-resident sweep (sgd_iteration), the medium-horizon one (sgd_iteration_q) or the segmented
-// adjoint (sgd_iteration_seg), with the same other-car slab; their per-thread buffers live in local memory here.
+// Phase 1 of both reverse kernels: re-run start s of problem b (world [C][4][B], weights w with stride ws, the start
+// built from `speed`) with the iteration code k_solve / k_episode run for this specialisation (HT, NOT_, LT, PRECISE):
+// the register-resident sweep (sgd_iteration), the medium-horizon one (sgd_iteration_q) or the segmented adjoint
+// (sgd_iteration_seg), with the same other-car slab; their per-thread buffers live in local memory here.  Stores
+// u^0 .. u^{N-1} (and u^N with store_last) to it [N (+1)][H][2] at element stride B; dead threads (live false) run
+// along without storing.
 template <int HT, int NOT_, int LT, bool PRECISE>
-__global__ void __launch_bounds__(kVjpThreads) k_solve_vjp(const __grid_constant__ KParams k, const VjpArgs a) {
+__device__ __forceinline__ void vjp_recompute(const KParams &k, const float *world, long long B, long long b, bool live,
+                                              const OtherControls &ocs_src, const float *w, int ws, int s, float speed,
+                                              float *it, bool store_last) {
     constexpr bool SEGK = (HT == 0) || OCD_IS_SEGC(HT, NOT_);
     constexpr bool QK = OCD_IS_Q(HT, NOT_) && !PRECISE;
-    const long long b_raw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const bool live = b_raw < a.B;
-    const long long b = live ? b_raw : a.B - 1;     // whole warps stay converged: the FAST feature code votes
-    const long long B = a.B;
     const bool lin = slab_is_linear(SEGK, PRECISE, k.other_mode, k.H, k.NO, QK);
     float oth[OCD_MAX_H * OCD_MAX_OTHER * 2];
-    for (int j = 0; j < k.NO; ++j) {
-        const float *st = a.world + (size_t)(j + 1) * 4 * B + b;
-        const float *oc = nullptr;
-        long long ocs = 0;
-        if (k.other_mode == 1) {
-            ocs = a.Bo;
-            oc = a.other_controls + (size_t)j * k.H * 2 * a.Bo + (a.Bo == 1 ? 0 : b);
+    {
+        float buf[2 * OCD_MAX_H];
+        for (int j = 0; j < k.NO; ++j) {
+            const float *st = world + (size_t)(j + 1) * 4 * B + b;
+            long long ocs;
+            const float *oc = ocs_src.car(k, j, b, buf, ocs);
+            predict_other<PRECISE>(k, st[0], st[B], st[2 * B], st[3 * B], oc, ocs, oth, j, 1, lin);
         }
-        predict_other<PRECISE>(k, st[0], st[B], st[2 * B], st[3 * B], oc, ocs, oth, j, 1, lin);
     }
-    const float *w = a.weights + weight_column(a.weight_idx, a.Bw, b);
-    const GradW gw = make_gradw<LT>(k, w, (int)a.Bw);
-    const float x0 = a.world[b], y0 = a.world[B + b], v0 = a.world[2 * B + b], th0 = a.world[3 * B + b];
-    int s = a.best[b];
-    s = s < 0 ? 0 : (s >= k.S ? k.S - 1 : s);
-    const float speed = a.cur_speed ? a.cur_speed[b] : v0;
+    const GradW gw = make_gradw<LT>(k, w, ws);
+    const float x0 = world[b], y0 = world[B + b], v0 = world[2 * B + b], th0 = world[3 * B + b];
     const int H = k.H;
-    float *it = a.iters + b;
+    const int n_store = k.n_iter + (store_last ? 1 : 0);
     if constexpr (SEGK) {
         constexpr int HC = HT;
         constexpr bool FR = HC > 0 && OCD_SEGC_FR && !PRECISE;
@@ -316,12 +361,13 @@ __global__ void __launch_bounds__(kVjpThreads) k_solve_vjp(const __grid_constant
             for (int t = 0; t < H; ++t) us.set(t, a0, w0);
         }
 #pragma unroll 1
-        for (int n = 0; n < k.n_iter; ++n) {
+        for (int n = 0; n < n_store; ++n) {
             if (live)
                 for (int t = 0; t < H; ++t) {
                     it[((size_t)(n * H + t) * 2 + 0) * B] = us.acc(t);
                     it[((size_t)(n * H + t) * 2 + 1) * B] = us.ang(t);
                 }
+            if (n == k.n_iter) break;
             if (!PRECISE && lin)
                 sgd_iteration_seg<SEGL, NOT_, LT, PRECISE, !PRECISE, 0, HC, FR>(k, gw, x0, y0, v0, th0, oth, 1, us,
                                                                               reinterpret_cast<float *>(ckbuf));
@@ -337,13 +383,14 @@ __global__ void __launch_bounds__(kVjpThreads) k_solve_vjp(const __grid_constant
         float4 q[QK ? HT : 1];
         float2 q2[QK ? HT : 1];                      // entry t at index t (t = 1 .. HT-1 are used)
 #pragma unroll 1
-        for (int n = 0; n < k.n_iter; ++n) {
+        for (int n = 0; n < n_store; ++n) {
             if (live)
 #pragma unroll
                 for (int t = 0; t < HT; ++t) {
                     it[((size_t)(n * HT + t) * 2 + 0) * B] = u.ua[t];
                     it[((size_t)(n * HT + t) * 2 + 1) * B] = u.uw[t];
                 }
+            if (n == k.n_iter) break;
             if constexpr (QK) {
                 if (lin) sgd_iteration_q<HT, NOT_, LT, 0, true>(k, gw, x0, y0, v0, th0, sn0, cs0, oth, 1, u, q, q2);
                 else sgd_iteration_q<HT, NOT_, LT, 0, false>(k, gw, x0, y0, v0, th0, sn0, cs0, oth, 1, u, q, q2);
@@ -353,6 +400,19 @@ __global__ void __launch_bounds__(kVjpThreads) k_solve_vjp(const __grid_constant
             }
         }
     }
+}
+
+template <int HT, int NOT_, int LT, bool PRECISE>
+__global__ void __launch_bounds__(kVjpThreads) k_solve_vjp(const __grid_constant__ KParams k, const VjpArgs a) {
+    const long long b_raw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = b_raw < a.B;
+    const long long b = live ? b_raw : a.B - 1;     // whole warps stay converged: the FAST feature code votes
+    int s = a.best[b];
+    s = s < 0 ? 0 : (s >= k.S ? k.S - 1 : s);
+    const float speed = a.cur_speed ? a.cur_speed[b] : a.world[2 * a.B + b];
+    vjp_recompute<HT, NOT_, LT, PRECISE>(k, a.world, a.B, b, live, OtherControls{a.other_controls, a.Bo, nullptr},
+                                         a.weights + weight_column(a.weight_idx, a.Bw, b), (int)a.Bw, s, speed,
+                                         a.iters + b, false);
     if (live) vjp_reverse(k, a, b, s);
 }
 
@@ -361,5 +421,176 @@ int launch_solve_vjp_t(const KParams &k, const VjpArgs &a, cudaStream_t st) {
     k_solve_vjp<HT, NOT_, LT, PRECISE><<<(unsigned)((a.B + kVjpThreads - 1) / kVjpThreads), kVjpThreads, 0, st>>>(k, a);
     return cuda_status();
 }
+
+// ---------------------------------------------------------------------------------------------
+// k_episode_vjp: the reverse pass through whole episodes (ocd_episode_vjp_batch).
+//
+// For world b, k_episode runs t = 0 .. T-1: world_t (after the replanning teleport; traj_states[t]), the reward
+// r_t = w_true . phi(world_t), the applied control u_t = pi(w, world_t) (the first control of the winning start
+// traj_best[t], planned from the robot's speed and the planner's model of the scripted cars), and the simulator step
+// s_{t+1} = f(s_t, clip(u_t)) of the robot.  The scripted cars depend on neither w nor the robot, so only the robot's
+// 4-state adjoint lambda is carried backwards from lambda_T = 0:
+//   ubar_t   = M_t (df/du)(s_t, u_t)^T lambda_{t+1}                      (M_t: the simulator's inclusive clip mask)
+//   lambda_t = ret_bar grad_s r_t + (df/ds)^T lambda_{t+1} + J_s,t^T ubar_t
+//   wbar    += J_w,t^T ubar_t
+// with J_t = d u_t / d(w, s_t) the 2 x (K + 4) Jacobian of the applied control: the solve VJP of step t seeded one-hot
+// on plan[0][0] and on plan[0][1].  Outputs: plan_weights_bar = wbar, robot_init_bar = lambda_0,
+// true_weights_bar = ret_bar sum_t phi(world_t).
+//
+// The steps' Jacobians are independent, so k_episode_jac runs one thread per (world, step) -- the step on
+// blockIdx.y -- and only the 4 x 4 chain is sequential (k_episode_adjoint, one thread per world).  k_episode_jac
+// re-runs step t's winning start with k_episode's own iteration code and other-car model (the episode dispatch:
+// OCD_DISPATCH, not the solve's compile-time horizons), stores u^0 .. u^N in the workspace -- u^N[0] is the applied
+// control, bit for bit traj_controls[t] -- and writes J_t to the workspace rows [T][2][K + 4][B].  The iterate store
+// ((N + 1) H 2 floats per world and step) bounds how many steps are in flight: the caller's workspace decides, from
+// one step per launch to all T; the results do not depend on it.
+// ---------------------------------------------------------------------------------------------
+struct EpisodeVjpArgs {
+    const float *plan_weights;     // [K][Bw]
+    long long    Bw;
+    const int32_t *weight_idx;     // [B] or null
+    const float *true_weights;     // [K]
+    int          T;
+    int          t0;               // first step of this k_episode_jac launch
+    const float *traj_states;      // [T][C][4][B]
+    const int32_t *traj_best;      // [T][B]
+    const float *traj_controls;    // [T][2][B]
+    const float *returns_bar;      // [B]
+    float       *plan_weights_bar; // [K][B]
+    float       *robot_init_bar;   // [4][B] or null
+    float       *true_weights_bar; // [K][B] or null
+    float       *jac;              // [T][2][K + 4][B] workspace
+    float       *iters;            // [steps in flight][N + 1][H][2][B] workspace
+    long long    B;
+};
+
+// The two reverse sweeps of (world b, step t): J_t rows for the seeds plan[0][0] and plan[0][1].
+static __device__ __noinline__ void episode_jac_reverse(const KParams &k, const ocd_scenario &sc,
+                                                        const EpisodeVjpArgs &a, const float *world, const float *it,
+                                                        long long b, int s, int t) {
+    const long long B = a.B;
+    const int H = k.H, NO = k.NO, KJ = k.K + 4;
+    float oth[OCD_MAX_H * OCD_MAX_OTHER * 2], obar[OCD_MAX_H * OCD_MAX_OTHER * 2];
+    vjp_predict_others(k, world, B, b, OtherControls{nullptr, 0, &sc}, oth);
+    const float s0[4] = {world[b], world[B + b], world[2 * B + b], world[3 * B + b]};
+    const float *w = a.plan_weights + weight_column(a.weight_idx, a.Bw, b);
+    const int ws = (int)a.Bw;
+    float *J = a.jac + (size_t)t * 2 * KJ * B + b;
+#pragma unroll 1
+    for (int c = 0; c < 2; ++c) {
+        float ubar[2 * OCD_MAX_H], wbar[kVjpK], s0bar[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+        for (int i = 0; i < 2 * H; ++i) ubar[i] = i == c ? 1.0f : 0.0f;
+        for (int i = 0; i < H * NO * 2; ++i) obar[i] = 0.0f;
+#pragma unroll
+        for (int q = 0; q < kVjpK; ++q) wbar[q] = 0.0f;
+        vjp_sweep(k, w, ws, s0, oth, it, B, s, true, ubar, wbar, s0bar, obar);
+#pragma unroll
+        for (int q = 0; q < kVjpK; ++q)
+            if (q < k.K) J[(size_t)(c * KJ + q) * B] = wbar[q];
+        for (int q = 0; q < 4; ++q) J[(size_t)(c * KJ + k.K + q) * B] = s0bar[q];
+    }
+}
+
+template <int HT, int NOT_, int LT, bool PRECISE>
+__global__ void __launch_bounds__(kVjpThreads)
+k_episode_jac(const __grid_constant__ KParams k, const __grid_constant__ ocd_scenario sc, const EpisodeVjpArgs a) {
+    const long long b_raw = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool live = b_raw < a.B;
+    const long long b = live ? b_raw : a.B - 1;     // whole warps stay converged: the FAST feature code votes
+    const long long B = a.B;
+    const int t = a.t0 + (int)blockIdx.y;
+    const float *world = a.traj_states + (size_t)t * (k.NO + 1) * 4 * B;
+    int s = a.traj_best[(size_t)t * B + b];
+    s = s < 0 ? 0 : (s >= k.S ? k.S - 1 : s);
+    float *it = a.iters + (size_t)blockIdx.y * (k.n_iter + 1) * k.H * 2 * B + b;
+    // k_episode plans from the robot's own speed (cur_speed = v0)
+    vjp_recompute<HT, NOT_, LT, PRECISE>(k, world, B, b, live, OtherControls{nullptr, 0, &sc},
+                                         a.plan_weights + weight_column(a.weight_idx, a.Bw, b), (int)a.Bw, s,
+                                         world[2 * B + b], it, true);
+    if (live) episode_jac_reverse(k, sc, a, world, it, b, s, t);
+}
+
+// k_episode_jac over the T steps, `group` steps per launch (1 .. T; the iterate store holds `group` steps)
+template <int HT, int NOT_, int LT, bool PRECISE>
+int launch_episode_jac_t(const KParams &k, const ocd_scenario &sc, const EpisodeVjpArgs &a, int group,
+                         cudaStream_t st) {
+    EpisodeVjpArgs g = a;
+    for (int t0 = 0; t0 < a.T; t0 += group) {
+        g.t0 = t0;
+        const dim3 grid((unsigned)((a.B + kVjpThreads - 1) / kVjpThreads), (unsigned)(a.T - t0 < group ? a.T - t0 : group));
+        k_episode_jac<HT, NOT_, LT, PRECISE><<<grid, kVjpThreads, 0, st>>>(k, sc, g);
+        const int rc = cuda_status();
+        if (rc) return rc;
+    }
+    return OCD_OK;
+}
+
+#ifndef OCD_HD_ONLY   // built once, by ocd_api.cu
+// The sequential part: one thread per world walks t = T-1 .. 0 with lambda and wbar in registers (precise arithmetic).
+// T = 0 writes zeros.
+__global__ void __launch_bounds__(kVjpThreads) k_episode_adjoint(const __grid_constant__ KParams k, const EpisodeVjpArgs a) {
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= a.B) return;
+    const long long B = a.B;
+    const int C = k.NO + 1, KJ = k.K + 4;
+    const float rb = a.T > 0 ? a.returns_bar[b] : 0.0f;
+    float lam[4] = {0.0f, 0.0f, 0.0f, 0.0f}, wbar[kVjpK], tbar[kVjpK], wt[kVjpK];
+#pragma unroll
+    for (int q = 0; q < kVjpK; ++q) {
+        wbar[q] = tbar[q] = 0.0f;
+        wt[q] = q < k.K ? a.true_weights[q] : 0.0f;
+    }
+    for (int t = a.T - 1; t >= 0; --t) {
+        const float *st = a.traj_states + (size_t)t * C * 4 * B + b;
+        const float x = st[0], y = st[B], v = st[2 * B], th = st[3 * B];
+        // the simulator step (dynamics_step with the robot's friction; clip masks inclusive, simulation_utils.py:9-21)
+        const float ua = a.traj_controls[(size_t)(2 * t) * B + b], uw = a.traj_controls[(size_t)(2 * t + 1) * B + b];
+        const float ac = fmaxf(fminf(ua, 4.0f), -8.0f);
+        const float sn = sinf(th), cs = cosf(th);
+        const float total = ac - k.mu * (v * v);
+        const float dist = v * k.dt + k.hdt2 * total;
+        const float ld = cs * lam[0] + sn * lam[1];               // adjoint of the step length
+        const float lt = k.hdt2 * ld + k.dt * lam[2];             // adjoint of the clipped acceleration
+        const float ub0 = (ua >= -8.0f && ua <= 4.0f) ? lt : 0.0f;
+        const float ub1 = fabsf(uw) <= 4.0f ? k.dt * lam[3] : 0.0f;
+        float nl[4] = {lam[0], lam[1], lam[2] + k.dt * ld - 2.0f * k.mu * v * lt, lam[3] + dist * (cs * lam[1] - sn * lam[0])};
+        // through the planner: u_t = pi(w, s_t)
+        const float *J = a.jac + (size_t)t * 2 * KJ * B + b;
+#pragma unroll
+        for (int q = 0; q < kVjpK; ++q)
+            if (q < k.K) wbar[q] = fmaf(ub0, J[(size_t)q * B], fmaf(ub1, J[(size_t)(KJ + q) * B], wbar[q]));
+        for (int i = 0; i < 4; ++i)
+            nl[i] = fmaf(ub0, J[(size_t)(k.K + i) * B], fmaf(ub1, J[(size_t)(KJ + k.K + i) * B], nl[i]));
+        // the reward of world_t, the other cars where they are
+        HD ox[OCD_MAX_OTHER], oy[OCD_MAX_OTHER];
+        for (int c = 0; c < k.NO; ++c) {
+            ox[c] = hd_const(st[(size_t)((c + 1) * 4) * B]);
+            oy[c] = hd_const(st[(size_t)((c + 1) * 4 + 1) * B]);
+        }
+        for (int i = 0; i < 4; ++i) {
+            HD phi[kVjpK];
+            hd_features(k, HD{x, i == 0 ? 1.0f : 0.0f, 0.0f, 0.0f}, HD{y, i == 1 ? 1.0f : 0.0f, 0.0f, 0.0f},
+                        HD{v, i == 2 ? 1.0f : 0.0f, 0.0f, 0.0f}, HD{th, i == 3 ? 1.0f : 0.0f, 0.0f, 0.0f}, ox, oy, phi);
+            float g = 0.0f;
+#pragma unroll
+            for (int q = 0; q < kVjpK; ++q)
+                if (q < k.K) {
+                    g = fmaf(wt[q], phi[q].a, g);
+                    if (i == 0) tbar[q] = fmaf(rb, phi[q].v, tbar[q]);
+                }
+            nl[i] = fmaf(rb, g, nl[i]);
+        }
+        for (int i = 0; i < 4; ++i) lam[i] = nl[i];
+    }
+#pragma unroll
+    for (int q = 0; q < kVjpK; ++q)
+        if (q < k.K) {
+            a.plan_weights_bar[(size_t)q * B + b] = wbar[q];
+            if (a.true_weights_bar) a.true_weights_bar[(size_t)q * B + b] = tbar[q];
+        }
+    if (a.robot_init_bar)
+        for (int i = 0; i < 4; ++i) a.robot_init_bar[(size_t)i * B + b] = lam[i];
+}
+#endif
 
 }  // namespace ocd

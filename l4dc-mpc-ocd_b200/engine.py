@@ -25,6 +25,8 @@ from . import _native as N
 
 MATH_FAST, MATH_PRECISE = 0, 1
 OPT_SGD, OPT_LBFGS = 0, 1
+# Engine.episodes_vjp_soa keeps every step's iterates in flight up to this many workspace bytes, fewer steps beyond
+EPISODE_VJP_WORKSPACE_CAP = 1 << 30
 
 
 @dataclass
@@ -300,6 +302,50 @@ class Engine:
                                          _ptr(out.get("controls")), _ptr(out.get("best")), _ptr(out.get("states")),
                                          _ptr(out.get("final_world")), B, self._stream())
         N.check(rc, "ocd_episode_batch")
+        self._kernel_launches += 1 if B else 0
+        return out
+
+    def episodes_vjp_soa(self, p: PlannerParams, sc: Scenario, plan_weights, Bw: int, true_weights, T: int, states,
+                         best, controls, returns_bar, weight_idx=None, robot_init_bar: bool = True,
+                         true_weights_bar: bool = True):
+        """Vector-Jacobian product of episodes_soa's returns (``ocd_episode_vjp_batch``): the same params, scenario,
+        plan_weights [K][Bw], weight_idx, true_weights [K] and T, the trace of that episode run (states [T][C][4][B],
+        best [T][B], controls [T][2][B]: episodes_soa(..., trace=True)) and returns_bar [B] = d loss / d returns ->
+        dict(plan_weights_bar [K][B], robot_init_bar [4][B], true_weights_bar [K][B]), rows per world (worlds sharing
+        a weight vector are not summed here).  The workspace holds the iterates of every step when that takes at most
+        EPISODE_VJP_WORKSPACE_CAP bytes, else of as many steps as fit (at least one); the results are the same."""
+        B = returns_bar.shape[-1]
+        dev = self.device
+        f32, i32 = torch.float32, torch.int32
+        _check_soa("plan_weights", plan_weights, f32, dev, (p.K, Bw))
+        _check_soa("true_weights", true_weights, f32, dev, (p.K,))
+        _check_soa("weight_idx", weight_idx, i32, dev, (B,))
+        _check_soa("states", states, f32, dev, (T, p.C, 4, B))
+        _check_soa("best", best, i32, dev, (T, B))
+        _check_soa("controls", controls, f32, dev, (T, 2, B))
+        _check_soa("returns_bar", returns_bar, f32, dev, (B,))
+        ps, ss = p.c_struct(), sc.c_struct()
+        lo, full = C.c_size_t(0), C.c_size_t(0)
+        N.check(N.lib.ocd_episode_vjp_workspace_bytes(C.addressof(ps), int(T), B, C.byref(lo), C.byref(full)),
+                "ocd_episode_vjp_workspace_bytes")
+        nbytes = full.value
+        if nbytes > EPISODE_VJP_WORKSPACE_CAP and T > 1:
+            step = (full.value - lo.value) // (T - 1)          # the iterates of one step
+            jac = lo.value - step
+            nbytes = jac + step * max(1, (EPISODE_VJP_WORKSPACE_CAP - jac) // step)
+        ws = torch.empty(((nbytes + 3) // 4,), dtype=f32, device=dev)
+        out = dict(plan_weights_bar=torch.empty((p.K, B), dtype=f32, device=dev))
+        if robot_init_bar:
+            out["robot_init_bar"] = torch.empty((4, B), dtype=f32, device=dev)
+        if true_weights_bar:
+            out["true_weights_bar"] = torch.empty((p.K, B), dtype=f32, device=dev)
+        with torch.cuda.device(dev):
+            rc = N.lib.ocd_episode_vjp_batch(C.addressof(ps), C.addressof(ss), _ptr(plan_weights), Bw, _ptr(weight_idx),
+                                             _ptr(true_weights), int(T), _ptr(states), _ptr(best), _ptr(controls),
+                                             _ptr(returns_bar), _ptr(out["plan_weights_bar"]),
+                                             _ptr(out.get("robot_init_bar")), _ptr(out.get("true_weights_bar")), _ptr(ws),
+                                             nbytes, B, self._stream())
+        N.check(rc, "ocd_episode_vjp_batch")
         self._kernel_launches += 1 if B else 0
         return out
 

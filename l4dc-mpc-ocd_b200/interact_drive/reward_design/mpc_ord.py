@@ -63,6 +63,21 @@ def _planning_weight_rows(W: np.ndarray) -> np.ndarray:
     return W.astype(np.float32)
 
 
+def _planning_weights_vjp(w: np.ndarray, g: np.ndarray) -> np.ndarray:
+    """The transposed Jacobian of MPC_ORD._planning_weights's three float64 normalisations at the raw vector w [K],
+    applied to g = d f / d (planning weights): -> d f / d w (float64; the final cast to float32 counts as the identity).
+    The normalisation x -> x / |x| has the Jacobian (I - u u^T) / |x|, u = x / |x|."""
+    xs = [np.asarray(w, dtype=np.float64)]
+    for _ in range(2):
+        xs.append(xs[-1] / math.sqrt(float(xs[-1].dot(xs[-1]))))
+    g = np.asarray(g, dtype=np.float64)
+    for x in reversed(xs):
+        n = math.sqrt(float(x.dot(x)))
+        u = x / n
+        g = (g - u * float(u.dot(g))) / n
+    return g
+
+
 def _launch_sharded(eng, ord_, W, robot, widx, unlucky):
     """One process per GPU: this rank runs its contiguous shard of the episodes, then the per-episode rows -- return
     and final world state -- are all-gathered (the path's only exchange step), so every rank holds the same data and
@@ -468,6 +483,38 @@ class MPC_ORD:
         if gif:
             raise NotImplementedError("gif rendering is outside the batched MPC engine's scope")
         return float(self.eval_weights_batch([weights])[0])
+
+    def eval_weights_grad(self, weights):
+        """-> (objective, grad): the objective is eval_weights(weights) bit for bit -- the same episode kernel on the same
+        batch, launched through the traced device path -- and grad its gradient with respect to the raw candidate
+        `weights` [K] (float64): the episodes' reverse pass (``ocd_episode_vjp_batch``) summed over the initial states
+        and samples, divided by the samples, through the three normalisations of _planning_weights.  History, iteration
+        counter and the replanning world's reset toggle advance exactly as in eval_weights, so the two can be mixed in
+        one optimisation."""
+        import torch
+        w = np.asarray(weights, dtype=np.float64)
+        w = w[0] if w.ndim == 2 else w
+        batch = self._episode_batch([w])
+        W, robot, widx, unlucky = batch["W"], batch["robot"], batch["widx"], batch["unlucky"]
+        p, sc, T = self.program.params, self.program.scenario, self.designer_horizon
+        eng = get_engine(self._device)
+        dev = eng.device
+        ri = torch.as_tensor(np.ascontiguousarray(robot.T), device=dev)
+        wp = torch.as_tensor(np.ascontiguousarray(W.T), device=dev)
+        tw = torch.as_tensor(as_f32(self.designer_weights), device=dev)
+        idx = torch.as_tensor(widx, device=dev)
+        ul = None if unlucky is None else torch.as_tensor(unlucky, device=dev)
+        out = eng.episodes_soa(p, sc, ri, wp, 1, tw, T, weight_idx=idx, unlucky_idx=ul, trace=True, final_world=True)
+        vjp = eng.episodes_vjp_soa(p, sc, wp, 1, tw, T, out["states"], out["best"], out["controls"],
+                                   torch.ones_like(out["returns"]), weight_idx=idx, robot_init_bar=False,
+                                   true_weights_bar=False)
+        ret = out["returns"].cpu().numpy()
+        self.kernel_launches += 1
+        self._after_episodes(batch, out["final_world"][:, :, -1].cpu().numpy())
+        objective = float(self._record([w], ret.reshape(batch["shape"]))[0])
+        # objective = -sum(returns) / num_samples
+        g_plan = -vjp["plan_weights_bar"].cpu().numpy().astype(np.float64).sum(axis=1) / self.num_samples
+        return objective, _planning_weights_vjp(w, g_plan)
 
     def eval_weights_batch(self, weight_matrix) -> np.ndarray:
         """eval_weights for every row of weight_matrix in ONE launch; history and iteration counter

@@ -1,6 +1,8 @@
 """The two planner entry points as PyTorch custom ops (``torch.ops.ocd_b200.solve`` /
-``torch.ops.ocd_b200.episodes``) and the reverse pass of the solve (``torch.ops.ocd_b200.solve_vjp``, which is
-also ``solve``'s autograd formula: gradients of the plan reach ``world`` and ``weights``): device tensors in,
+``torch.ops.ocd_b200.episodes``) and their reverse passes (``torch.ops.ocd_b200.solve_vjp``, which is also
+``solve``'s autograd formula: gradients of the plan reach ``world`` and ``weights``; ``torch.ops.ocd_b200.episodes_vjp``
+with ``episodes_trace``, ``episodes``' autograd formula: gradients of the returns reach ``robot_init``,
+``plan_weights`` and ``true_weights``): device tensors in,
 device tensors out, launched on the current stream through the same C ABI as everything else.  Registering them makes the engine usable from code that
 composes torch ops (and gives them fake-tensor shape functions); there is deliberately no CPU kernel --
 calling them with CPU tensors is an error, not a fallback.
@@ -138,6 +140,82 @@ def episodes(robot_init: torch.Tensor, plan_weights: torch.Tensor, weight_idx: O
 @episodes.register_fake
 def _(robot_init, plan_weights, weight_idx, true_weights, unlucky_idx, params, scenario, T):
     return robot_init.new_empty((robot_init.shape[-1],))
+
+
+@torch.library.custom_op("ocd_b200::episodes_trace", mutates_args=())
+def episodes_trace(robot_init: torch.Tensor, plan_weights: torch.Tensor, weight_idx: Optional[torch.Tensor],
+                   true_weights: torch.Tensor, unlucky_idx: Optional[torch.Tensor], params: List[float],
+                   scenario: List[float], T: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor, torch.Tensor]:
+    """episodes with its per-step trace -> (returns [B], controls [T,2,B], best [T,B] i32, states [T,C,4,B]): the same
+    kernel and the same bits as episodes; what episodes_vjp differentiates along."""
+    p = unpack_params(params)
+    sc = unpack_scenario(scenario)
+    eng = _engine(robot_init)
+    out = eng.episodes_soa(p, sc, robot_init.contiguous(), plan_weights.contiguous(), plan_weights.shape[-1],
+                           true_weights.contiguous(), int(T),
+                           weight_idx=None if weight_idx is None else weight_idx.contiguous(),
+                           unlucky_idx=None if unlucky_idx is None else unlucky_idx.contiguous(), trace=True)
+    return out["returns"], out["controls"], out["best"], out["states"]
+
+
+@episodes_trace.register_fake
+def _(robot_init, plan_weights, weight_idx, true_weights, unlucky_idx, params, scenario, T):
+    p = unpack_params(params)
+    B = robot_init.shape[-1]
+    return (robot_init.new_empty((B,)), robot_init.new_empty((T, 2, B)),
+            robot_init.new_empty((T, B), dtype=torch.int32), robot_init.new_empty((T, p.C, 4, B)))
+
+
+@torch.library.custom_op("ocd_b200::episodes_vjp", mutates_args=())
+def episodes_vjp(plan_weights: torch.Tensor, weight_idx: Optional[torch.Tensor], true_weights: torch.Tensor,
+                 states: torch.Tensor, best: torch.Tensor, controls: torch.Tensor, returns_bar: torch.Tensor,
+                 params: List[float], scenario: List[float], T: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """episodes' inputs, the trace of that run (episodes_trace) and returns_bar [B] = d loss / d returns ->
+    (plan_weights_bar [K,B]: per world, d loss / d the weight vector world b planned with; robot_init_bar [4,B];
+    true_weights_bar [K,B]: per world)."""
+    p = unpack_params(params)
+    sc = unpack_scenario(scenario)
+    eng = _engine(states)
+    out = eng.episodes_vjp_soa(p, sc, plan_weights.contiguous(), plan_weights.shape[-1], true_weights.contiguous(),
+                               int(T), states.contiguous(), best.contiguous(), controls.contiguous(),
+                               returns_bar.contiguous(), None if weight_idx is None else weight_idx.contiguous())
+    return out["plan_weights_bar"], out["robot_init_bar"], out["true_weights_bar"]
+
+
+@episodes_vjp.register_fake
+def _(plan_weights, weight_idx, true_weights, states, best, controls, returns_bar, params, scenario, T):
+    p = unpack_params(params)
+    B = returns_bar.shape[-1]
+    return returns_bar.new_empty((p.K, B)), returns_bar.new_empty((4, B)), returns_bar.new_empty((p.K, B))
+
+
+def _episodes_setup_context(ctx, inputs, output):
+    robot_init, plan_weights, weight_idx, true_weights, unlucky_idx, params, scenario, T = inputs
+    ctx.save_for_backward(robot_init, plan_weights, weight_idx, true_weights, unlucky_idx)
+    ctx.params, ctx.scenario, ctx.T = params, scenario, T
+
+
+def _episodes_backward(ctx, returns_bar):
+    robot_init, plan_weights, weight_idx, true_weights, unlucky_idx = ctx.saved_tensors
+    # the trace of the forward's own run: the same kernel on the same inputs, so the same bits
+    _, controls, best, states = torch.ops.ocd_b200.episodes_trace(robot_init, plan_weights, weight_idx, true_weights,
+                                                                  unlucky_idx, ctx.params, ctx.scenario, ctx.T)
+    pw_bar, ri_bar, tw_bar = torch.ops.ocd_b200.episodes_vjp(plan_weights, weight_idx, true_weights, states, best,
+                                                            controls, returns_bar.contiguous(), ctx.params,
+                                                            ctx.scenario, ctx.T)
+    Bw, B = plan_weights.shape[-1], robot_init.shape[-1]
+    if weight_idx is not None:
+        # rows of the worlds that share a vector, summed deterministically (see _solve_backward)
+        wb = torch.zeros((Bw, pw_bar.shape[0]), dtype=pw_bar.dtype, device=pw_bar.device)
+        wb.index_put_((weight_idx.long(),), pw_bar.t(), accumulate=True)
+        pw_bar = wb.t()
+    elif Bw == 1 and B != 1:
+        pw_bar = pw_bar.sum(dim=1, keepdim=True)
+    return (ri_bar if ctx.needs_input_grad[0] else None, pw_bar if ctx.needs_input_grad[1] else None, None,
+            tw_bar.sum(dim=1) if ctx.needs_input_grad[3] else None, None, None, None, None)
+
+
+episodes.register_autograd(_episodes_backward, setup_context=_episodes_setup_context)
 
 
 def pack_scenario(sc: Scenario) -> List[float]:
