@@ -205,6 +205,24 @@ int ocd_solve_vjp_batch(const ocd_params *p, const float *world /*[C][4][B]*/,
                         float *weights_bar /*[K][B]*/, float *world_bar /*[C][4][B] or NULL*/,
                         void *workspace, size_t workspace_bytes, int64_t B, void *stream);
 
+/* Vector-Jacobian product of the L-BFGS plan (optimizer == 1: k_solve_lbfgs, ocd_api.cu) with respect to the weights
+ * and the initial world, by the implicit function theorem at the plan: with A the controls inside the inclusive clip
+ * box, G = d reward / d controls and H = dG/d controls, solve H_AA z_A = plan_bar_A (z = 0 on the clipped controls),
+ * then (weights_bar, world_bar) = -grad_(w, world) (G . z).  It is the derivative of the optimum the plan stands for:
+ * exact where the plan is stationary (G_A = 0), and whatever the line search, restarts and the start did to reach it.
+ * A clipped control has zero derivative.  A singular H_AA (a pivot below the float rounding of its entries) gives
+ * NaN weights_bar and world_bar for that problem alone.  Inputs as for ocd_solve_batch, plus its plan [H][2][B] for
+ * the same inputs; cur_speed does not enter.  world_bar and residual may be NULL.  Nothing is summed across
+ * problems.  optimizer == 0 -> OCD_EUNSUP (ocd_solve_vjp_batch differentiates the SGD plan exactly).
+ * Outputs: weights_bar [K][B], world_bar [C][4][B], residual [B] = max over A of |G| at the plan (its stationarity). */
+int ocd_solve_implicit_vjp_batch(const ocd_params *p, const float *world /*[C][4][B]*/,
+                                 const float *other_controls, int64_t Bo,
+                                 const float *weights, int64_t Bw, const int32_t *weight_idx,
+                                 const float *plan /*[H][2][B], from ocd_solve_batch*/,
+                                 const float *plan_bar /*[H][2][B]*/,
+                                 float *weights_bar /*[K][B]*/, float *world_bar /*[C][4][B] or NULL*/,
+                                 float *residual /*[B] or NULL*/, int64_t B, void *stream);
+
 /* The receding-horizon episode of MPC_ORD.eval_weights_for_init
  * (interact_drive/reward_design/mpc_ord.py:87-103): T times CarWorld.step
  * (interact_drive/world.py:79-109; ReplanningCarWorld.step experiments/replanning_world.py:29-36),

@@ -741,6 +741,25 @@ int ocd_solve_vjp_batch(const ocd_params *p, const float *world, const float *ot
     return launch_solve_vjp(k, p->math_mode == 1, a, (cudaStream_t)stream);
 }
 
+int ocd_solve_implicit_vjp_batch(const ocd_params *p, const float *world, const float *other_controls, int64_t Bo,
+                                 const float *weights, int64_t Bw, const int32_t *weight_idx, const float *plan,
+                                 const float *plan_bar, float *weights_bar, float *world_bar, float *residual,
+                                 int64_t B, void *stream) {
+    KParams k;
+    int rc = digest(p, k);
+    if (rc) return rc;
+    if (k.optimizer != 1) return OCD_EUNSUP;      // the SGD plan has the exact unrolled derivative (ocd_solve_vjp_batch)
+    if (B == 0) return OCD_OK;
+    if (!world || !plan || !plan_bar || !weights_bar || B < 0) return OCD_EINVAL;
+    if ((rc = check_weights(weights, Bw, weight_idx, B))) return rc;
+    if (k.other_mode == 1 && (!other_controls || (Bo != 1 && Bo != B))) return OCD_EINVAL;
+    const ImplicitVjpArgs a{world, other_controls, Bo, weights, Bw, weight_idx, plan, plan_bar, weights_bar, world_bar,
+                            residual, B};
+    k_solve_implicit_vjp<<<(unsigned)((B + kVjpThreads - 1) / kVjpThreads), kVjpThreads, 0, (cudaStream_t)stream>>>(k,
+                                                                                                                  a);
+    return cuda_status();
+}
+
 int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc, const float *robot_init,
                       const float *other_init, const float *plan_weights, int64_t Bw,
                       const int32_t *weight_idx, const float *true_weights, const int32_t *unlucky_idx,

@@ -29,8 +29,11 @@
 //
 // The second half of the file is the reverse pass through whole episodes (ocd_episode_vjp_batch): the same recompute
 // phase and reverse sweep per (world, step), seeded on the applied control, then the robot's adjoint along the episode
-// (see k_episode_vjp below).
+// (see k_episode_vjp below).  The file ends with the implicit-function derivative of the L-BFGS plan
+// (ocd_solve_implicit_vjp_batch: k_solve_implicit_vjp), built from the same forward-over-reverse sweep.
 #pragma once
+
+#include <cfloat>
 
 #include "ocd_kernels.cuh"
 #include "ocd_hessian.cuh"
@@ -134,12 +137,14 @@ __device__ __forceinline__ void grad_and_tangent(const KParams &k, const float *
     }
 }
 
-// One iteration of the reverse pass at the iterate u = u^n ([2H], flat index 2t + c).  On entry ubar holds ubar^{n+1},
-// on exit ubar^n; wbar [K], s0bar [4] (robot) and obar [H][NO][2] (the other cars' predicted positions) gain
-// lr * grad phi_n.  oth: the predicted positions [H][NO][2] (precise).
-__device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, int ws, const float (&s0)[4],
-                                              const float *oth, const float *u, float *ubar, float *wbar,
-                                              float *s0bar, float *obar) {
+// One forward-over-reverse sweep at the controls u ([2H], flat index 2t + c) along the direction d ([2H]): hv gets
+// the Hessian-vector product M H M d (zero on the clipped controls), and with GRADS wbar [K], s0bar [4] (robot) and
+// obar [H][NO][2] (the other cars' predicted positions) gain scale * the gradients of G(u) . M d with respect to the
+// weights, the robot's initial state and the predicted positions.  oth: the predicted positions [H][NO][2] (precise).
+template <bool GRADS>
+__device__ __forceinline__ void vjp_hvp(const KParams &k, const float *w, int ws, const float (&s0)[4],
+                                        const float *oth, const float *u, const float *d, float *hv, float scale,
+                                        float *wbar, float *s0bar, float *obar) {
     const int H = k.H;
     float S[OCD_MAX_H + 1][4], Sd[OCD_MAX_H + 1][4], D[OCD_MAX_H], Dd[OCD_MAX_H];
     for (int q = 0; q < 4; ++q) {
@@ -151,7 +156,7 @@ __device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, 
         const float a = u[2 * t], om = u[2 * t + 1];
         const bool in_a = (a >= -8.0f) && (a <= 4.0f), in_w = fabsf(om) <= 4.0f;
         const float ac = fmaxf(fminf(a, 4.0f), -8.0f), oc = fmaxf(fminf(om, 4.0f), -4.0f);
-        const float acd = in_a ? ubar[2 * t] : 0.0f, ocd = in_w ? ubar[2 * t + 1] : 0.0f;
+        const float acd = in_a ? d[2 * t] : 0.0f, ocd = in_w ? d[2 * t + 1] : 0.0f;
         const float x = S[t][0], y = S[t][1], v = S[t][2], th = S[t][3];
         const float xd = Sd[t][0], yd = Sd[t][1], vd = Sd[t][2], thd = Sd[t][3];
         const float sn = sinf(th), cs = cosf(th), snd = cs * thd, csd = -sn * thd;
@@ -175,10 +180,13 @@ __device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, 
         const float st[4] = {S[t + 1][0], S[t + 1][1], S[t + 1][2], S[t + 1][3]};
         const float sdt[4] = {Sd[t + 1][0], Sd[t + 1][1], Sd[t + 1][2], Sd[t + 1][3]};
         grad_and_tangent(k, w, ws, st, sdt, oth + (size_t)t * k.NO * 2, g, gd, phid);
+        if constexpr (GRADS) {
 #pragma unroll
-        for (int q = 0; q < kVjpK; ++q)
-            if (q < k.K) wbar[q] = fmaf(k.lr, phid[q], wbar[q]);
-        for (int c = 0; c < 2 * k.NO; ++c) obar[(size_t)t * k.NO * 2 + c] = fmaf(k.lr, gd[4 + c], obar[(size_t)t * k.NO * 2 + c]);
+            for (int q = 0; q < kVjpK; ++q)
+                if (q < k.K) wbar[q] = fmaf(scale, phid[q], wbar[q]);
+            for (int c = 0; c < 2 * k.NO; ++c)
+                obar[(size_t)t * k.NO * 2 + c] = fmaf(scale, gd[4 + c], obar[(size_t)t * k.NO * 2 + c]);
+        }
         const float mx = g[0] + lx, my = g[1] + ly, mv = g[2] + lv, mth = g[3] + lth;
         const float mxd = gd[0] + lxd, myd = gd[1] + lyd, mvd = gd[2] + lvd, mthd = gd[3] + lthd;
         const float v = S[t][2], vd = Sd[t][2], th = S[t][3], thd = Sd[t][3];
@@ -195,13 +203,29 @@ __device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, 
         lthd = mthd + Dd[t] * cr + D[t] * crd;
         lx = mx; ly = my; lxd = mxd; lyd = myd;
         const float a = u[2 * t], om = u[2 * t + 1];
-        if ((a >= -8.0f) && (a <= 4.0f)) ubar[2 * t] = fmaf(k.lr, ltd, ubar[2 * t]);
-        if (fabsf(om) <= 4.0f) ubar[2 * t + 1] = fmaf(k.lr, k.dt * mthd, ubar[2 * t + 1]);
+        hv[2 * t] = ((a >= -8.0f) && (a <= 4.0f)) ? ltd : 0.0f;
+        hv[2 * t + 1] = (fabsf(om) <= 4.0f) ? k.dt * mthd : 0.0f;
     }
-    s0bar[0] = fmaf(k.lr, lxd, s0bar[0]);
-    s0bar[1] = fmaf(k.lr, lyd, s0bar[1]);
-    s0bar[2] = fmaf(k.lr, lvd, s0bar[2]);
-    s0bar[3] = fmaf(k.lr, lthd, s0bar[3]);
+    if constexpr (GRADS) {
+        s0bar[0] = fmaf(scale, lxd, s0bar[0]);
+        s0bar[1] = fmaf(scale, lyd, s0bar[1]);
+        s0bar[2] = fmaf(scale, lvd, s0bar[2]);
+        s0bar[3] = fmaf(scale, lthd, s0bar[3]);
+    }
+}
+
+// One iteration of the reverse pass at the iterate u = u^n: on entry ubar holds ubar^{n+1}, on exit
+// ubar^n = ubar^{n+1} + lr M H M ubar^{n+1}; wbar, s0bar and obar gain lr * grad phi_n.
+__device__ __forceinline__ void vjp_iteration(const KParams &k, const float *w, int ws, const float (&s0)[4],
+                                              const float *oth, const float *u, float *ubar, float *wbar,
+                                              float *s0bar, float *obar) {
+    float hv[2 * OCD_MAX_H];
+    vjp_hvp<true>(k, w, ws, s0, oth, u, ubar, hv, k.lr, wbar, s0bar, obar);
+    for (int t = 0; t < k.H; ++t) {
+        const float a = u[2 * t], om = u[2 * t + 1];
+        if ((a >= -8.0f) && (a <= 4.0f)) ubar[2 * t] = fmaf(k.lr, hv[2 * t], ubar[2 * t]);
+        if (fabsf(om) <= 4.0f) ubar[2 * t + 1] = fmaf(k.lr, hv[2 * t + 1], ubar[2 * t + 1]);
+    }
 }
 
 // Where the planner's model of the other cars takes its known controls from (other_mode == 1): a solve's
@@ -242,6 +266,45 @@ __device__ __forceinline__ void vjp_predict_others(const KParams &k, const float
         long long ocs;
         const float *oc = ocs_src.car(k, j, b, buf, ocs);
         predict_other<true>(k, st[0], st[B], st[2 * B], st[3 * B], oc, ocs, oth, j, 1);
+    }
+}
+
+// The other cars' rows of world_bar [C][4][B]: obar [H][NO][2], the gradient with respect to the predicted positions,
+// chained through the prediction model (naive_planner.py:53-66; known controls or constant velocity) in forward
+// mode, one seed per component of car j's initial state.
+__device__ __forceinline__ void vjp_chain_others(const KParams &k, const float *world, long long B, long long b,
+                                                 const OtherControls &ocs_src, const float *obar, float *world_bar) {
+    const int H = k.H, NO = k.NO;
+    float buf[2 * OCD_MAX_H];
+    for (int j = 0; j < NO; ++j) {
+        const float *st = world + (size_t)(j + 1) * 4 * B + b;
+        long long ocs;
+        const float *oc = ocs_src.car(k, j, b, buf, ocs);
+        for (int q = 0; q < 4; ++q) {
+            float x = st[0], y = st[B], v = st[2 * B], th = st[3 * B];
+            float xd = q == 0, yd = q == 1, vd = q == 2, thd = q == 3;
+            float acc = 0.0f;
+            for (int t = 0; t < H; ++t) {
+                const float sn = sinf(th), cs = cosf(th);
+                if (oc) {
+                    const float oa = oc[(size_t)(t * 2 + 0) * ocs], oo = oc[(size_t)(t * 2 + 1) * ocs];
+                    const float dist = v * k.dt + 0.5f * oa * k.dt2, distd = vd * k.dt;
+                    x += cs * dist;
+                    y += sn * dist;
+                    xd += -sn * thd * dist + cs * distd;
+                    yd += cs * thd * dist + sn * distd;
+                    v += oa * k.dt;
+                    th += oo * k.dt;
+                } else {
+                    x += cs * v * k.dt;
+                    y += sn * v * k.dt;
+                    xd += (cs * vd - sn * thd * v) * k.dt;
+                    yd += (sn * vd + cs * thd * v) * k.dt;
+                }
+                acc = fmaf(obar[(size_t)(t * NO + j) * 2], xd, fmaf(obar[(size_t)(t * NO + j) * 2 + 1], yd, acc));
+            }
+            world_bar[(size_t)((j + 1) * 4 + q) * B + b] = acc;
+        }
     }
 }
 
@@ -287,37 +350,7 @@ static __device__ __noinline__ void vjp_reverse(const KParams &k, const VjpArgs 
         if (q < k.K) a.weights_bar[(size_t)q * B + b] = wbar[q];
     if (!a.world_bar) return;
     for (int q = 0; q < 4; ++q) a.world_bar[(size_t)q * B + b] = s0bar[q];
-    // other car j: obar through the prediction model (naive_planner.py:53-66) in forward mode, one seed per component
-    for (int j = 0; j < NO; ++j) {
-        const float *st = a.world + (size_t)(j + 1) * 4 * B + b;
-        const float *oc = (k.other_mode == 1) ? a.other_controls + (size_t)j * H * 2 * a.Bo + (a.Bo == 1 ? 0 : b)
-                                              : nullptr;
-        for (int q = 0; q < 4; ++q) {
-            float x = st[0], y = st[B], v = st[2 * B], th = st[3 * B];
-            float xd = q == 0, yd = q == 1, vd = q == 2, thd = q == 3;
-            float acc = 0.0f;
-            for (int t = 0; t < H; ++t) {
-                const float sn = sinf(th), cs = cosf(th);
-                if (oc) {
-                    const float oa = oc[(size_t)(t * 2 + 0) * a.Bo], oo = oc[(size_t)(t * 2 + 1) * a.Bo];
-                    const float dist = v * k.dt + 0.5f * oa * k.dt2, distd = vd * k.dt;
-                    x += cs * dist;
-                    y += sn * dist;
-                    xd += -sn * thd * dist + cs * distd;
-                    yd += cs * thd * dist + sn * distd;
-                    v += oa * k.dt;
-                    th += oo * k.dt;
-                } else {
-                    x += cs * v * k.dt;
-                    y += sn * v * k.dt;
-                    xd += (cs * vd - sn * thd * v) * k.dt;
-                    yd += (sn * vd + cs * thd * v) * k.dt;
-                }
-                acc = fmaf(obar[(size_t)(t * NO + j) * 2], xd, fmaf(obar[(size_t)(t * NO + j) * 2 + 1], yd, acc));
-            }
-            a.world_bar[(size_t)((j + 1) * 4 + q) * B + b] = acc;
-        }
-    }
+    vjp_chain_others(k, a.world, B, b, ocs_src, obar, a.world_bar);
 }
 
 // Phase 1 of both reverse kernels: re-run start s of problem b (world [C][4][B], weights w with stride ws, the start
@@ -590,6 +623,143 @@ __global__ void __launch_bounds__(kVjpThreads) k_episode_adjoint(const __grid_co
         }
     if (a.robot_init_bar)
         for (int i = 0; i < 4; ++i) a.robot_init_bar[(size_t)i * B + b] = lam[i];
+}
+// ---------------------------------------------------------------------------------------------
+// k_solve_implicit_vjp: the implicit-function derivative of the L-BFGS plan (ocd_solve_implicit_vjp_batch).
+//
+// k_solve_lbfgs returns a stationary point u* of R: with A the controls inside the inclusive clip box at u* (the
+// forward's masks) and G = dR/du (zero on the clipped controls), G_A(u*; theta) = 0 for theta = (w, s0).  The
+// implicit function theorem gives du*_A/dtheta = -H_AA^{-1} dG_A/dtheta (H = dG/du) and du*_I/dtheta = 0 for the
+// clipped controls I, so with z_A the solution of H_AA z_A = plan_bar_A (z_I = 0)
+//   theta_bar = -grad_theta (G(u*; theta) . z).
+// The line search, restarts and early breaks of the run that found u* do not enter, and neither do the start it began
+// from nor cur_speed.  One thread per problem, precise arithmetic: |A| sweeps of vjp_hvp along the unit vectors of A
+// give the columns of H_AA, which is symmetrised and solved in double with partial pivoting; a pivot that vanishes
+// relative to the largest entry (below the float rounding of the entries) marks the problem singular and its
+// weights_bar and world_bar are NaN.  One more sweep along z with scale -1 gives weights_bar, the robot's world_bar
+// and obar, which vjp_chain_others carries to the other cars.  residual (optional) = max_A |G(u*)|, from the
+// gradient code k_solve_lbfgs itself runs: the stationarity the derivative assumes.
+// ---------------------------------------------------------------------------------------------
+struct ImplicitVjpArgs {
+    const float *world;            // [C][4][B]
+    const float *other_controls;   // [NO][H][2][Bo] or null
+    long long    Bo;
+    const float *weights;          // [K][Bw]
+    long long    Bw;
+    const int32_t *weight_idx;     // [B] or null
+    const float *plan;             // [H][2][B] (ocd_solve_batch's, optimizer 1)
+    const float *plan_bar;         // [H][2][B]
+    float       *weights_bar;      // [K][B]
+    float       *world_bar;        // [C][4][B] or null
+    float       *residual;         // [B] or null
+    long long    B;
+};
+
+static constexpr int kImplicitN = 2 * OCD_LBFGS_MAX_H;
+
+__global__ void __launch_bounds__(kVjpThreads) k_solve_implicit_vjp(const __grid_constant__ KParams k,
+                                                                    const ImplicitVjpArgs a) {
+    const long long b = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= a.B) return;
+    const long long B = a.B;
+    const int H = k.H, n = 2 * k.H;
+    const OtherControls ocs_src{a.other_controls, a.Bo, nullptr};
+    float oth[OCD_LBFGS_MAX_H * OCD_MAX_OTHER * 2], obar[OCD_LBFGS_MAX_H * OCD_MAX_OTHER * 2];
+    vjp_predict_others(k, a.world, B, b, ocs_src, oth);
+    for (int i = 0; i < H * k.NO * 2; ++i) obar[i] = 0.0f;
+    const float s0[4] = {a.world[b], a.world[B + b], a.world[2 * B + b], a.world[3 * B + b]};
+    const float *w = a.weights + weight_column(a.weight_idx, a.Bw, b);
+    const int ws = (int)a.Bw;
+    float u[kImplicitN], d[kImplicitN], hv[kImplicitN];
+    int act[kImplicitN];
+    int na = 0;
+    for (int t = 0; t < H; ++t) {
+        const float ua = a.plan[(size_t)(2 * t) * B + b], uw = a.plan[(size_t)(2 * t + 1) * B + b];
+        u[2 * t] = ua;
+        u[2 * t + 1] = uw;
+        if ((ua >= -8.0f) && (ua <= 4.0f)) act[na++] = 2 * t;
+        if (fabsf(uw) <= 4.0f) act[na++] = 2 * t + 1;
+    }
+    if (a.residual) {
+        Traj<0> ut;
+        float ga[OCD_MAX_H], go[OCD_MAX_H], sn0, cs0;
+        for (int t = 0; t < H; ++t) {
+            ut.ua[t] = u[2 * t];
+            ut.uw[t] = u[2 * t + 1];
+        }
+        Mth<true>::sincos_(s0[3], sn0, cs0);
+        sgd_iteration<0, 0, 0, true, false>(k, make_gradw<0>(k, w, ws), s0[0], s0[1], s0[2], s0[3], sn0, cs0, oth, 1,
+                                            ut, ga, go);
+        float r = 0.0f;
+        for (int t = 0; t < H; ++t) r = fmaxf(r, fmaxf(fabsf(ga[t]), fabsf(go[t])));   // zero on the clipped controls
+        a.residual[b] = r;
+    }
+    // H_AA, column by column, then symmetrised (row-major, n_A x n_A)
+    double M[kImplicitN * kImplicitN], z[kImplicitN];
+    for (int i = 0; i < n; ++i) d[i] = 0.0f;
+    for (int j = 0; j < na; ++j) {
+        d[act[j]] = 1.0f;
+        vjp_hvp<false>(k, w, ws, s0, oth, u, d, hv, 0.0f, nullptr, nullptr, nullptr);
+        d[act[j]] = 0.0f;
+        for (int i = 0; i < na; ++i) M[i * na + j] = (double)hv[act[i]];
+    }
+    double scale = 0.0;
+    for (int i = 0; i < na; ++i) {
+        for (int j = 0; j < i; ++j) {
+            const double m = 0.5 * (M[i * na + j] + M[j * na + i]);
+            M[i * na + j] = M[j * na + i] = m;
+        }
+        for (int j = 0; j < na; ++j) scale = fmax(scale, fabs(M[i * na + j]));
+        z[i] = (double)a.plan_bar[(size_t)act[i] * B + b];
+    }
+    // Gaussian elimination with partial pivoting.  The entries carry float rounding, so a pivot below na float ulps
+    // of the largest entry cannot be told apart from zero: the reduced Hessian is singular there.
+    const double tiny = (double)na * (double)FLT_EPSILON * scale;
+    bool singular = false;
+    for (int c = 0; c < na && !singular; ++c) {
+        int piv = c;
+        for (int r = c + 1; r < na; ++r)
+            if (fabs(M[r * na + c]) > fabs(M[piv * na + c])) piv = r;
+        if (!(fabs(M[piv * na + c]) > tiny)) {
+            singular = true;
+            break;
+        }
+        if (piv != c) {
+            for (int j = c; j < na; ++j) {
+                const double t = M[c * na + j]; M[c * na + j] = M[piv * na + j]; M[piv * na + j] = t;
+            }
+            const double t = z[c]; z[c] = z[piv]; z[piv] = t;
+        }
+        for (int r = c + 1; r < na; ++r) {
+            const double f = M[r * na + c] / M[c * na + c];
+            for (int j = c + 1; j < na; ++j) M[r * na + j] -= f * M[c * na + j];
+            z[r] -= f * z[c];
+        }
+    }
+    if (singular) {
+        const float nan = __int_as_float(0x7fffffff);
+        for (int q = 0; q < k.K; ++q) a.weights_bar[(size_t)q * B + b] = nan;
+        if (a.world_bar)
+            for (int q = 0; q < (k.NO + 1) * 4; ++q) a.world_bar[(size_t)q * B + b] = nan;
+        return;
+    }
+    for (int r = na - 1; r >= 0; --r) {
+        double acc = z[r];
+        for (int j = r + 1; j < na; ++j) acc -= M[r * na + j] * z[j];
+        z[r] = acc / M[r * na + r];
+    }
+    // theta_bar = -grad_theta (G . z): one sweep along z with scale -1
+    for (int i = 0; i < na; ++i) d[act[i]] = (float)z[i];
+    float wbar[kVjpK], s0bar[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+    for (int q = 0; q < kVjpK; ++q) wbar[q] = 0.0f;
+    vjp_hvp<true>(k, w, ws, s0, oth, u, d, hv, -1.0f, wbar, s0bar, obar);
+#pragma unroll
+    for (int q = 0; q < kVjpK; ++q)
+        if (q < k.K) a.weights_bar[(size_t)q * B + b] = wbar[q];
+    if (!a.world_bar) return;
+    for (int q = 0; q < 4; ++q) a.world_bar[(size_t)q * B + b] = s0bar[q];
+    vjp_chain_others(k, a.world, B, b, ocs_src, obar, a.world_bar);
 }
 #endif
 

@@ -1,5 +1,6 @@
 """The two planner entry points as PyTorch custom ops (``torch.ops.ocd_b200.solve`` /
-``torch.ops.ocd_b200.episodes``) and their reverse passes (``torch.ops.ocd_b200.solve_vjp``, which is also
+``torch.ops.ocd_b200.episodes``) and their reverse passes (``torch.ops.ocd_b200.solve_vjp`` for SGD plans and
+``torch.ops.ocd_b200.solve_implicit_vjp`` for L-BFGS plans, which make up
 ``solve``'s autograd formula: gradients of the plan reach ``world`` and ``weights``; ``torch.ops.ocd_b200.episodes_vjp``
 with ``episodes_trace``, ``episodes``' autograd formula: gradients of the returns reach ``robot_init``,
 ``plan_weights`` and ``true_weights``): device tensors in,
@@ -86,10 +87,32 @@ def _(world, weights, weight_idx, other_controls, best, plan_bar, params):
     return world.new_empty((p.K, B)), world.new_empty((p.C, 4, B))
 
 
+@torch.library.custom_op("ocd_b200::solve_implicit_vjp", mutates_args=())
+def solve_implicit_vjp(world: torch.Tensor, weights: torch.Tensor, weight_idx: Optional[torch.Tensor],
+                       other_controls: Optional[torch.Tensor], plan: torch.Tensor, plan_bar: torch.Tensor,
+                       params: List[float]) -> Tuple[torch.Tensor, torch.Tensor]:
+    """solve's inputs with L-BFGS params, its plan [H,2,B] and plan_bar [H,2,B] = d loss / d plan -> (weights_bar [K,B]:
+    per problem; world_bar [C,4,B]): the implicit-function derivative of the optimum the plan stands for."""
+    p = unpack_params(params)
+    eng = _engine(world)
+    Bo = 0 if other_controls is None else other_controls.shape[-1]
+    out = eng.solve_implicit_vjp_soa(p, world.contiguous(), weights.contiguous(), weights.shape[-1], plan.contiguous(),
+                                     plan_bar.contiguous(), None if weight_idx is None else weight_idx.contiguous(),
+                                     None if other_controls is None else other_controls.contiguous(), Bo)
+    return out["weights_bar"], out["world_bar"]
+
+
+@solve_implicit_vjp.register_fake
+def _(world, weights, weight_idx, other_controls, plan, plan_bar, params):
+    p = unpack_params(params)
+    B = world.shape[-1]
+    return world.new_empty((p.K, B)), world.new_empty((p.C, 4, B))
+
+
 def _solve_setup_context(ctx, inputs, output):
     world, weights, weight_idx, other_controls, params = inputs
     ctx.set_materialize_grads(False)          # an output nobody differentiates arrives as None, not as zeros
-    ctx.save_for_backward(world, weights, weight_idx, other_controls, output[2])
+    ctx.save_for_backward(world, weights, weight_idx, other_controls, output[2], output[0])
     ctx.params = params
 
 
@@ -100,11 +123,16 @@ def _solve_backward(ctx, plan_bar, losses_bar, best_bar):
     if ctx.needs_input_grad[3]:
         raise RuntimeError("ocd_b200::solve: gradients with respect to other_controls are not supported; "
                            "pass other_controls without requires_grad")
-    world, weights, weight_idx, other_controls, best = ctx.saved_tensors
+    world, weights, weight_idx, other_controls, best, plan = ctx.saved_tensors
     if plan_bar is None:
         return None, None, None, None, None
-    weights_bar, world_bar = torch.ops.ocd_b200.solve_vjp(world, weights, weight_idx, other_controls, best,
-                                                          plan_bar.contiguous(), ctx.params)
+    if unpack_params(ctx.params).optimizer == 1:
+        # L-BFGS: the derivative of the optimum the plan stands for (the line search is not differentiated)
+        weights_bar, world_bar = torch.ops.ocd_b200.solve_implicit_vjp(world, weights, weight_idx, other_controls,
+                                                                       plan, plan_bar.contiguous(), ctx.params)
+    else:
+        weights_bar, world_bar = torch.ops.ocd_b200.solve_vjp(world, weights, weight_idx, other_controls, best,
+                                                              plan_bar.contiguous(), ctx.params)
     Bw, B = weights.shape[-1], world.shape[-1]
     if weight_idx is not None:
         # rows of the problems that share a vector, summed deterministically: index_put_ with accumulate=True sorts by
