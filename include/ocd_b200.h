@@ -239,7 +239,11 @@ int ocd_solve_implicit_vjp_batch(const ocd_params *p, const float *world /*[C][4
  *   returns      [B]   sum over the T steps of true_weights . features(past_state)
  *   traj_controls [T][2][B], traj_best [T][B], traj_states [T][C][4][B] (past states): optional
  *   final_world  [C][4][B] optional: world state after the last step
- * With T == 1 this is exactly one CarWorld.step for B worlds. */
+ * With T == 1 this is exactly one CarWorld.step for B worlds.
+ * With params.optimizer == 1 every step plans with the L-BFGS planner (k_episode_lbfgs, precise math whatever
+ * math_mode): step t is ocd_solve_batch (optimizer 1) on traj_states[t] bit for bit, with other_controls = the
+ * scenario's controls (a fixed-plan car's plan from index 0, zero for the other scripted cars) and cur_speed = the
+ * robot's speed. */
 int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc,
                       const float *robot_init, const float *other_init,
                       const float *plan_weights, int64_t Bw, const int32_t *weight_idx,
@@ -271,6 +275,32 @@ int ocd_episode_vjp_batch(const ocd_params *p, const ocd_scenario *sc,
                           float *plan_weights_bar /*[K][B]*/, float *robot_init_bar /*[4][B] or NULL*/,
                           float *true_weights_bar /*[K][B] or NULL*/,
                           void *workspace, size_t workspace_bytes, int64_t B, void *stream);
+
+/* Vector-Jacobian product of ocd_episode_batch's returns for the L-BFGS planner (optimizer == 1; optimizer 0 ->
+ * OCD_EUNSUP, ocd_episode_vjp_batch differentiates the SGD planner).  Arguments and outputs as for
+ * ocd_episode_vjp_batch.  Each step's control Jacobian is the implicit-function derivative of the optimum at that step
+ * (as in ocd_solve_implicit_vjp_batch): the step's winning start is re-run, the reduced Hessian H_AA of the controls
+ * inside the clip box is built, and it is solved in double for the two first-control seeds.  Controls whose row and
+ * column of H_AA are exactly zero (decoupled: their gradient vanishes in a neighbourhood) and controls whose
+ * curvature is below the float rounding of H_AA (after equilibration and elimination with diagonal pivoting) are held
+ * at their value, z = 0: the planner does not move them either.  A clipped first control has a zero row; a held one
+ * keeps its start value, whose only dependence is friction * speed^2 of the extra-init accelerations.  A matrix the
+ * elimination cannot factor (a remaining diagonal below the rounding beside a larger off-diagonal) makes that world's
+ * outputs NaN and leaves the others unaffected.  The steps run in parallel, one launch for all T.  workspace: device
+ * memory of at least ocd_episode_implicit_vjp_workspace_bytes() bytes, laid out as the Jacobian rows [T][2][K + 4][B],
+ * the recomputed plans [T][H][2][B] (the plan of step t's winning start; its first control is traj_controls[t] bit
+ * for bit), the status [T][B] (float: the number of held controls, -1 where the step is singular) and the held
+ * controls [T][B] (uint32 bit mask, bit 2t + c for control c of step t).  Too small -> OCD_EINVAL.  T == 0 writes
+ * zeros. */
+int ocd_episode_implicit_vjp_workspace_bytes(const ocd_params *p, int32_t T, int64_t B, size_t *bytes);
+int ocd_episode_implicit_vjp_batch(const ocd_params *p, const ocd_scenario *sc,
+                                   const float *plan_weights, int64_t Bw, const int32_t *weight_idx,
+                                   const float *true_weights, int32_t T,
+                                   const float *traj_states /*[T][C][4][B]*/, const int32_t *traj_best /*[T][B]*/,
+                                   const float *traj_controls /*[T][2][B]*/, const float *returns_bar /*[B]*/,
+                                   float *plan_weights_bar /*[K][B]*/, float *robot_init_bar /*[4][B] or NULL*/,
+                                   float *true_weights_bar /*[K][B] or NULL*/,
+                                   void *workspace, size_t workspace_bytes, int64_t B, void *stream);
 
 /* ---- host-buffer convenience layer (what a Python/ctypes caller without torch uses) ---------
  * An ocd_ctx owns a device, a stream, pinned staging buffers and device buffers that grow on

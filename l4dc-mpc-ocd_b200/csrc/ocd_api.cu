@@ -20,6 +20,7 @@
 #include "ocd_kernels.cuh"
 #include "ocd_hessian.cuh"
 #include "ocd_vjp.cuh"
+#include "ocd_lbfgs.cuh"
 
 namespace ocd {
 
@@ -160,35 +161,10 @@ k_dynamics(const float *state, const float *control, float dt, float dt2, float 
 
 // ---------------------------------------------------------------------------------------------
 // k_solve_lbfgs -- the opt-in L-BFGS optimiser (params.optimizer == 1; include/ocd_b200.h).
-// Same block shape, slab and argmin as k_solve; per (problem, start) the thread runs L-BFGS on
-// f(u) = -R(u): two-loop recursion over 4 correction pairs held in local memory, Armijo backtracking,
-// gradient from the same closed-form adjoint.  Lanes of a warp take different numbers of line-search
-// trials, so the warp-voting FAST feature code cannot be used here: the kernel always runs the precise
-// math path.  The CPU restatement used by the parity tests mirrors this loop statement for statement.
+// Same block shape, slab and argmin as k_solve; per (problem, start) the thread runs lbfgs_start (ocd_lbfgs.cuh).
+// Lanes of a warp take different numbers of line-search trials, so the warp-voting FAST feature code cannot be used
+// here: the kernel always runs the precise math path.
 // ---------------------------------------------------------------------------------------------
-static constexpr int kLbfgsM = 4, kLbfgsLS = 6, kLbfgsN = 2 * OCD_LBFGS_MAX_H;
-
-__device__ __forceinline__ float lbfgs_value_grad(const KParams &k, const GradW &gw, const float *wraw, int ws, float x0,
-                                                  float y0, float v0, float th0, const float *oth, int P,
-                                                  const float *uf, float *g /* null: value only */) {
-    Traj<0> u;
-    for (int t = 0; t < k.H; ++t) {
-        u.ua[t] = uf[2 * t];
-        u.uw[t] = uf[2 * t + 1];
-    }
-    const float f = -rollout_reward<0, 0, true>(k, wraw, ws, x0, y0, v0, th0, oth, P, u);
-    if (g) {
-        float ga[OCD_MAX_H], go[OCD_MAX_H], sn0, cs0;
-        Mth<true>::sincos_(th0, sn0, cs0);
-        sgd_iteration<0, 0, 0, true, false>(k, gw, x0, y0, v0, th0, sn0, cs0, oth, P, u, ga, go);
-        for (int t = 0; t < k.H; ++t) {            // gradient of f = -R
-            g[2 * t] = -ga[t];
-            g[2 * t + 1] = -go[t];
-        }
-    }
-    return f;
-}
-
 __global__ void __launch_bounds__(kMaxThreads) k_solve_lbfgs(const __grid_constant__ KParams k, const SolveArgs a) {
     extern __shared__ __align__(16) float smem_raw[];
     constexpr int P = kP;
@@ -215,100 +191,10 @@ __global__ void __launch_bounds__(kMaxThreads) k_solve_lbfgs(const __grid_consta
     __syncthreads();
     const float x0 = a.world[b], y0 = a.world[B + b], v0 = a.world[2 * B + b], th0 = a.world[3 * B + b];
     const GradW gw = make_gradw<0>(k, m.wraw + p, P);
-    const float *wraw = m.wraw + p, *oth = m.oth + p;
     const int n = 2 * k.H;
-    float u[kLbfgsN], g[kLbfgsN], gt[kLbfgsN], d[kLbfgsN], ut[kLbfgsN], q[kLbfgsN];
-    float Sh[kLbfgsM][kLbfgsN], Yh[kLbfgsM][kLbfgsN], rho[kLbfgsM], al[kLbfgsM];
-    {
-        const float speed = a.cur_speed ? a.cur_speed[b] : v0;
-        const float a0 = (s >= 3) ? __fmul_rn(k.mu, __fmul_rn(speed, speed)) : 0.0f;
-        const int mm = s % 3;
-        const float w0 = (mm == 0) ? 0.0f : ((mm == 1) ? -k.turn : k.turn);
-        for (int t = 0; t < k.H; ++t) {
-            u[2 * t] = a0;
-            u[2 * t + 1] = w0;
-        }
-    }
-    float f = lbfgs_value_grad(k, gw, wraw, P, x0, y0, v0, th0, oth, P, u, g);
-    float sy_last = 0.0f, yy_last = 1.0f;
-    int kk = 0, head = 0;
-    for (int it = 0; it < k.n_iter; ++it) {
-        for (int j = 0; j < n; ++j) q[j] = g[j];
-        for (int i = 0; i < kk; ++i) {                      // newest pair first
-            const int idx = (head - 1 - i + 2 * kLbfgsM) % kLbfgsM;
-            float dot = 0.0f;
-            for (int j = 0; j < n; ++j) dot = __fadd_rn(dot, __fmul_rn(Sh[idx][j], q[j]));
-            al[i] = __fmul_rn(rho[idx], dot);
-            for (int j = 0; j < n; ++j) q[j] = __fsub_rn(q[j], __fmul_rn(al[i], Yh[idx][j]));
-        }
-        {
-            const float gamma = (kk > 0) ? __fdiv_rn(sy_last, yy_last) : k.lr;
-            for (int j = 0; j < n; ++j) q[j] = __fmul_rn(gamma, q[j]);
-        }
-        for (int i = kk - 1; i >= 0; --i) {                 // oldest pair first
-            const int idx = (head - 1 - i + 2 * kLbfgsM) % kLbfgsM;
-            float dot = 0.0f;
-            for (int j = 0; j < n; ++j) dot = __fadd_rn(dot, __fmul_rn(Yh[idx][j], q[j]));
-            const float bb = __fmul_rn(rho[idx], dot);
-            for (int j = 0; j < n; ++j) q[j] = __fadd_rn(q[j], __fmul_rn(Sh[idx][j], __fsub_rn(al[i], bb)));
-        }
-        float gd = 0.0f;
-        for (int j = 0; j < n; ++j) {
-            d[j] = -q[j];
-            gd = __fadd_rn(gd, __fmul_rn(g[j], d[j]));
-        }
-        if (!(gd < 0.0f)) {                                 // not a descent direction: restart
-            kk = 0;
-            gd = 0.0f;
-            for (int j = 0; j < n; ++j) {
-                d[j] = __fmul_rn(-k.lr, g[j]);
-                gd = __fadd_rn(gd, __fmul_rn(g[j], d[j]));
-            }
-        }
-        if (!(gd < 0.0f)) break;
-        float t = 1.0f, ft = f;
-        bool ok = false;
-        for (int ls = 0; ls < kLbfgsLS; ++ls) {
-            for (int j = 0; j < n; ++j) ut[j] = __fadd_rn(u[j], __fmul_rn(t, d[j]));
-            ft = lbfgs_value_grad(k, gw, wraw, P, x0, y0, v0, th0, oth, P, ut, nullptr);
-            if (ft <= __fadd_rn(f, __fmul_rn(__fmul_rn(1e-4f, t), gd))) {
-                ok = true;
-                break;
-            }
-            t = __fmul_rn(t, 0.5f);
-        }
-        if (!ok) break;
-        lbfgs_value_grad(k, gw, wraw, P, x0, y0, v0, th0, oth, P, ut, gt);
-        {
-            // the candidate pair goes to scratch (d and q are free here): once the ring is full, slot `head` holds the
-            // oldest pair the two-loop recursion still reads, and a rejected candidate must not overwrite it
-            float sy = 0.0f, yy = 0.0f;
-            for (int j = 0; j < n; ++j) {
-                const float sj = __fsub_rn(ut[j], u[j]), yj = __fsub_rn(gt[j], g[j]);
-                d[j] = sj;
-                q[j] = yj;
-                sy = __fadd_rn(sy, __fmul_rn(sj, yj));
-                yy = __fadd_rn(yy, __fmul_rn(yj, yj));
-            }
-            if (yy > 0.0f && sy > __fmul_rn(1e-10f, yy)) {
-                for (int j = 0; j < n; ++j) {
-                    Sh[head][j] = d[j];
-                    Yh[head][j] = q[j];
-                }
-                rho[head] = __fdiv_rn(1.0f, sy);
-                head = (head + 1) % kLbfgsM;
-                if (kk < kLbfgsM) ++kk;
-                sy_last = sy;
-                yy_last = yy;
-            }
-        }
-        for (int j = 0; j < n; ++j) {
-            u[j] = ut[j];
-            g[j] = gt[j];
-        }
-        f = ft;
-    }
-    const float loss = lbfgs_value_grad(k, gw, wraw, P, x0, y0, v0, th0, oth, P, u, nullptr);
+    float u[kLbfgsN];
+    const float loss = lbfgs_start(k, gw, m.wraw + p, P, x0, y0, v0, th0, m.oth + p, P, s,
+                                   a.cur_speed ? a.cur_speed[b] : v0, u);
     m.loss[s * P + p] = loss;
     if (live) {
         a.losses[(size_t)s * B + b] = loss;
@@ -568,7 +454,7 @@ int ocd_kernel_form(const ocd_params *p, int64_t B, int episode) {
     const int rc = digest(p, k);
     if (rc) return rc;
     if (B < 0) return OCD_EINVAL;
-    if (k.optimizer == 1) return episode ? (int)OCD_EUNSUP : (int)OCD_FORM_THROUGHPUT;     // k_solve_lbfgs has one form
+    if (k.optimizer == 1) return OCD_FORM_THROUGHPUT;     // k_solve_lbfgs and k_episode_lbfgs have one form each
     return form_of(k, p->math_mode == 1, B, episode != 0);
 }
 
@@ -771,7 +657,6 @@ int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc, const float *
     if (B == 0) return OCD_OK;
     if (!sc || !robot_init || !true_weights || !returns || B < 0 || T < 0 || t0 < 0) return OCD_EINVAL;
     if (sc->n_other != k.NO) return OCD_EINVAL;
-    if (k.optimizer != 0) return OCD_EUNSUP;      // the episode loop runs the reference's SGD planner only
     for (int j = 0; j < k.NO; ++j)
         if (sc->plan_len[j] < 0 || sc->plan_len[j] > OCD_MAX_PLAN || (sc->kind[j] != 0 && sc->kind[j] != 1))
             return OCD_EINVAL;
@@ -779,6 +664,12 @@ int ocd_episode_batch(const ocd_params *p, const ocd_scenario *sc, const float *
     if (B == 0) return OCD_OK;
     EpisodeArgs a{robot_init, other_init, plan_weights, Bw, weight_idx, true_weights, unlucky_idx, t0, T,
                   returns, traj_controls, traj_best, traj_states, final_world, B, pick_P(B)};
+    if (k.optimizer == 1) {
+        const size_t bytes = smem_floats(k.H, k.NO, k.K, k.S, kP, true, false, false) * sizeof(float);
+        if ((rc = prepare_smem(k_episode_lbfgs, bytes))) return rc;
+        k_episode_lbfgs<<<(unsigned)((B + kP - 1) / kP), k.S * kP, bytes, (cudaStream_t)stream>>>(k, *sc, a);
+        return cuda_status();
+    }
     return launch_episode(k, p->math_mode == 1, *sc, a, (cudaStream_t)stream);
 }
 
@@ -834,6 +725,60 @@ int ocd_episode_vjp_batch(const ocd_params *p, const ocd_scenario *sc, const flo
         if (group > 65535) group = 65535;
         if ((rc = launch_episode_jac(k, p->math_mode == 1, *sc, a, (int)group, st))) return rc;
     }
+    k_episode_adjoint<<<(unsigned)((B + kVjpThreads - 1) / kVjpThreads), kVjpThreads, 0, st>>>(k, a);
+    return cuda_status();
+}
+
+// workspace of ocd_episode_implicit_vjp_batch: the Jacobian rows [T][2][K + 4][B], the recomputed plans [T][H][2][B],
+// the per-step status [T][B] (float) and held-control masks [T][B] (uint32)
+static size_t episode_implicit_bytes(const KParams &k, int32_t T, int64_t B) {
+    return episode_jac_bytes(k, T, B) + (size_t)T * ((size_t)k.H * 2 + 2) * (size_t)B * sizeof(float);
+}
+
+int ocd_episode_implicit_vjp_workspace_bytes(const ocd_params *p, int32_t T, int64_t B, size_t *bytes) {
+    KParams k;
+    const int rc = digest(p, k);
+    if (rc) return rc;
+    if (!bytes || B < 0 || T < 0) return OCD_EINVAL;
+    if (k.optimizer != 1) return OCD_EUNSUP;      // the SGD planner has the unrolled derivative (ocd_episode_vjp_batch)
+    *bytes = episode_implicit_bytes(k, T, B);
+    return OCD_OK;
+}
+
+int ocd_episode_implicit_vjp_batch(const ocd_params *p, const ocd_scenario *sc, const float *plan_weights, int64_t Bw,
+                                   const int32_t *weight_idx, const float *true_weights, int32_t T,
+                                   const float *traj_states, const int32_t *traj_best, const float *traj_controls,
+                                   const float *returns_bar, float *plan_weights_bar, float *robot_init_bar,
+                                   float *true_weights_bar, void *workspace, size_t workspace_bytes, int64_t B,
+                                   void *stream) {
+    KParams k;
+    int rc = digest(p, k);
+    if (rc) return rc;
+    if (k.optimizer != 1) return OCD_EUNSUP;
+    if (B == 0) return OCD_OK;
+    if (!sc || !true_weights || !returns_bar || !plan_weights_bar || B < 0 || T < 0) return OCD_EINVAL;
+    if (T > 0 && (!traj_states || !traj_best || !traj_controls)) return OCD_EINVAL;
+    if (sc->n_other != k.NO) return OCD_EINVAL;
+    for (int j = 0; j < k.NO; ++j)
+        if (sc->plan_len[j] < 0 || sc->plan_len[j] > OCD_MAX_PLAN || (sc->kind[j] != 0 && sc->kind[j] != 1))
+            return OCD_EINVAL;
+    if ((rc = check_weights(plan_weights, Bw, weight_idx, B))) return rc;
+    const size_t need = episode_implicit_bytes(k, T, B);
+    if (workspace_bytes < need || (need > 0 && !workspace)) return OCD_EINVAL;
+    float *jac = static_cast<float *>(workspace);
+    float *plans = jac + (size_t)T * 2 * (k.K + 4) * B;
+    float *status = plans + (size_t)T * k.H * 2 * B;
+    EpisodeImplicitArgs ja{plan_weights, Bw, weight_idx, 0, traj_states, traj_best, jac, plans, status,
+                           reinterpret_cast<unsigned *>(status + (size_t)T * B), B};
+    const cudaStream_t st = (cudaStream_t)stream;
+    for (int t0 = 0; t0 < T; t0 += 65535) {       // gridDim.y
+        ja.t0 = t0;
+        const dim3 grid((unsigned)((B + kVjpThreads - 1) / kVjpThreads), (unsigned)(T - t0 < 65535 ? T - t0 : 65535));
+        k_episode_jac_implicit<<<grid, kVjpThreads, 0, st>>>(k, *sc, ja);
+        if ((rc = cuda_status())) return rc;
+    }
+    EpisodeVjpArgs a{plan_weights, Bw, weight_idx, true_weights, T, 0, traj_states, traj_best, traj_controls,
+                     returns_bar, plan_weights_bar, robot_init_bar, true_weights_bar, jac, nullptr, B};
     k_episode_adjoint<<<(unsigned)((B + kVjpThreads - 1) / kVjpThreads), kVjpThreads, 0, st>>>(k, a);
     return cuda_status();
 }

@@ -383,6 +383,54 @@ class Engine:
         self._kernel_launches += 1 if B else 0
         return out
 
+    def episodes_implicit_vjp_soa(self, p: PlannerParams, sc: Scenario, plan_weights, Bw: int, true_weights, T: int,
+                                  states, best, controls, returns_bar, weight_idx=None, robot_init_bar: bool = True,
+                                  true_weights_bar: bool = True, details: bool = False):
+        """Vector-Jacobian product of episodes_soa's returns for the L-BFGS planner (p.optimizer == OPT_LBFGS), by the
+        implicit function theorem at every step's plan (``ocd_episode_implicit_vjp_batch``): arguments and outputs as
+        for episodes_vjp_soa.  A world with a singular step gets NaN rows.  With details=True the output also holds
+        the workspace: the control Jacobians jac [T][2][K + 4][B] (d first control / d (weights, robot state) of every
+        step), the recomputed plans [T][H][2][B] (the plan of every step's winning start), status [T][B] (the
+        number of controls the step holds at their value, -1 where it is singular) and held [T][B] (int32 bit mask
+        of those controls, bit 2t + c; bit 31 reads as the sign)."""
+        B = returns_bar.shape[-1]
+        dev = self.device
+        f32, i32 = torch.float32, torch.int32
+        _check_soa("plan_weights", plan_weights, f32, dev, (p.K, Bw))
+        _check_soa("true_weights", true_weights, f32, dev, (p.K,))
+        _check_soa("weight_idx", weight_idx, i32, dev, (B,))
+        _check_soa("states", states, f32, dev, (T, p.C, 4, B))
+        _check_soa("best", best, i32, dev, (T, B))
+        _check_soa("controls", controls, f32, dev, (T, 2, B))
+        _check_soa("returns_bar", returns_bar, f32, dev, (B,))
+        ps, ss = p.c_struct(), sc.c_struct()
+        nbytes = C.c_size_t(0)
+        N.check(N.lib.ocd_episode_implicit_vjp_workspace_bytes(C.addressof(ps), int(T), B, C.byref(nbytes)),
+                "ocd_episode_implicit_vjp_workspace_bytes")
+        ws = torch.empty((nbytes.value // 4,), dtype=f32, device=dev)
+        out = dict(plan_weights_bar=torch.empty((p.K, B), dtype=f32, device=dev))
+        if robot_init_bar:
+            out["robot_init_bar"] = torch.empty((4, B), dtype=f32, device=dev)
+        if true_weights_bar:
+            out["true_weights_bar"] = torch.empty((p.K, B), dtype=f32, device=dev)
+        with torch.cuda.device(dev):
+            rc = N.lib.ocd_episode_implicit_vjp_batch(C.addressof(ps), C.addressof(ss), _ptr(plan_weights), Bw,
+                                                      _ptr(weight_idx), _ptr(true_weights), int(T), _ptr(states),
+                                                      _ptr(best), _ptr(controls), _ptr(returns_bar),
+                                                      _ptr(out["plan_weights_bar"]), _ptr(out.get("robot_init_bar")),
+                                                      _ptr(out.get("true_weights_bar")), _ptr(ws), nbytes.value, B,
+                                                      self._stream())
+        N.check(rc, "ocd_episode_implicit_vjp_batch")
+        self._kernel_launches += 1 if B else 0
+        if details:
+            jac = T * 2 * (p.K + 4) * B
+            out["jac"] = ws[:jac].view(T, 2, p.K + 4, B)
+            out["plans"] = ws[jac:jac + T * p.H * 2 * B].view(T, p.H, 2, B)
+            st = jac + T * p.H * 2 * B
+            out["status"] = ws[st:st + T * B].view(T, B)
+            out["held"] = ws[st + T * B:st + 2 * T * B].view(torch.int32).view(T, B)
+        return out
+
     # -- natural-shape entry points ------------------------------------------------------------
     def _world(self, p: PlannerParams, world) -> torch.Tensor:
         w = torch.as_tensor(world, dtype=torch.float32, device=self.device)

@@ -8,6 +8,7 @@ one launch of the episode kernel (`ocd_episode_batch`); the Python world is only
 POD description the kernel needs."""
 from __future__ import annotations
 
+import dataclasses
 import pickle
 import sys
 import time
@@ -19,6 +20,7 @@ import numpy as np
 import scipy.stats
 
 from ... import cmaes as _cma
+from ... import engine as _eng
 from ... import parallel as _par
 from ...batched import compile_world, unlucky_sequence
 from ...experiments.merging import ThreeLaneCarWorld, ThreeLaneTestCar
@@ -284,7 +286,11 @@ class MPC_ORD:
     the receding-horizon episodes it produces."""
 
     def __init__(self, world, car, init_car_states, designer_horizon, save_path=None, num_samples=1, *,
-                 verbose: bool = True, device: Optional[int] = None):
+                 verbose: bool = True, device: Optional[int] = None, planner_optimizer: int = _eng.OPT_SGD,
+                 planner_iters: Optional[int] = None):
+        """planner_optimizer=OPT_LBFGS has every episode plan with the L-BFGS planner (precise math, H <= 16) instead of
+        the car's SGD planner, for eval_weights, eval_weights_batch, the CMA-ES loops and eval_weights_grad alike;
+        planner_iters replaces the planner's iteration budget (n_iter; L-BFGS: the maximum number of iterations)."""
         self.world, self.car = world, car
         self.designer_horizon = designer_horizon
         self.init_car_states = init_car_states
@@ -305,6 +311,10 @@ class MPC_ORD:
         self.verbose = verbose
         self._device = device
         self.program = compile_world(world, car)
+        if planner_optimizer != _eng.OPT_SGD or planner_iters is not None:
+            self.program.params = dataclasses.replace(
+                self.program.params, optimizer=int(planner_optimizer),
+                n_iter=self.program.params.n_iter if planner_iters is None else int(planner_iters))
         self.kernel_launches = 0
         self._dev_cache = {}
         self._batch_cache = None
@@ -487,7 +497,8 @@ class MPC_ORD:
     def eval_weights_grad(self, weights):
         """-> (objective, grad): the objective is eval_weights(weights) bit for bit -- the same episode kernel on the same
         batch, launched through the traced device path -- and grad its gradient with respect to the raw candidate
-        `weights` [K] (float64): the episodes' reverse pass (``ocd_episode_vjp_batch``) summed over the initial states
+        `weights` [K] (float64): the episodes' reverse pass (``ocd_episode_vjp_batch``; with the L-BFGS planner
+        ``ocd_episode_implicit_vjp_batch``) summed over the initial states
         and samples, divided by the samples, through the three normalisations of _planning_weights.  History, iteration
         counter and the replanning world's reset toggle advance exactly as in eval_weights, so the two can be mixed in
         one optimisation."""
@@ -505,9 +516,11 @@ class MPC_ORD:
         idx = torch.as_tensor(widx, device=dev)
         ul = None if unlucky is None else torch.as_tensor(unlucky, device=dev)
         out = eng.episodes_soa(p, sc, ri, wp, 1, tw, T, weight_idx=idx, unlucky_idx=ul, trace=True, final_world=True)
-        vjp = eng.episodes_vjp_soa(p, sc, wp, 1, tw, T, out["states"], out["best"], out["controls"],
-                                   torch.ones_like(out["returns"]), weight_idx=idx, robot_init_bar=False,
-                                   true_weights_bar=False)
+        # L-BFGS planner: every step's control Jacobian by the implicit function theorem at its plan
+        episodes_vjp = eng.episodes_implicit_vjp_soa if p.optimizer == _eng.OPT_LBFGS else eng.episodes_vjp_soa
+        vjp = episodes_vjp(p, sc, wp, 1, tw, T, out["states"], out["best"], out["controls"],
+                           torch.ones_like(out["returns"]), weight_idx=idx, robot_init_bar=False,
+                           true_weights_bar=False)
         ret = out["returns"].cpu().numpy()
         self.kernel_launches += 1
         self._after_episodes(batch, out["final_world"][:, :, -1].cpu().numpy())

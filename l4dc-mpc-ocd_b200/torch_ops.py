@@ -2,7 +2,8 @@
 ``torch.ops.ocd_b200.episodes``) and their reverse passes (``torch.ops.ocd_b200.solve_vjp`` for SGD plans and
 ``torch.ops.ocd_b200.solve_implicit_vjp`` for L-BFGS plans, which make up
 ``solve``'s autograd formula: gradients of the plan reach ``world`` and ``weights``; ``torch.ops.ocd_b200.episodes_vjp``
-with ``episodes_trace``, ``episodes``' autograd formula: gradients of the returns reach ``robot_init``,
+(SGD) or ``torch.ops.ocd_b200.episodes_implicit_vjp`` (L-BFGS) with ``episodes_trace``, ``episodes``' autograd formula:
+gradients of the returns reach ``robot_init``,
 ``plan_weights`` and ``true_weights``): device tensors in,
 device tensors out, launched on the current stream through the same C ABI as everything else.  Registering them makes the engine usable from code that
 composes torch ops (and gives them fake-tensor shape functions); there is deliberately no CPU kernel --
@@ -217,6 +218,30 @@ def _(plan_weights, weight_idx, true_weights, states, best, controls, returns_ba
     return returns_bar.new_empty((p.K, B)), returns_bar.new_empty((4, B)), returns_bar.new_empty((p.K, B))
 
 
+@torch.library.custom_op("ocd_b200::episodes_implicit_vjp", mutates_args=())
+def episodes_implicit_vjp(plan_weights: torch.Tensor, weight_idx: Optional[torch.Tensor], true_weights: torch.Tensor,
+                          states: torch.Tensor, best: torch.Tensor, controls: torch.Tensor, returns_bar: torch.Tensor,
+                          params: List[float], scenario: List[float],
+                          T: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """episodes_vjp for L-BFGS params: every step's control Jacobian by the implicit function theorem at its plan
+    -> (plan_weights_bar [K,B], robot_init_bar [4,B], true_weights_bar [K,B]), per world."""
+    p = unpack_params(params)
+    sc = unpack_scenario(scenario)
+    eng = _engine(states)
+    out = eng.episodes_implicit_vjp_soa(p, sc, plan_weights.contiguous(), plan_weights.shape[-1],
+                                        true_weights.contiguous(), int(T), states.contiguous(), best.contiguous(),
+                                        controls.contiguous(), returns_bar.contiguous(),
+                                        None if weight_idx is None else weight_idx.contiguous())
+    return out["plan_weights_bar"], out["robot_init_bar"], out["true_weights_bar"]
+
+
+@episodes_implicit_vjp.register_fake
+def _(plan_weights, weight_idx, true_weights, states, best, controls, returns_bar, params, scenario, T):
+    p = unpack_params(params)
+    B = returns_bar.shape[-1]
+    return returns_bar.new_empty((p.K, B)), returns_bar.new_empty((4, B)), returns_bar.new_empty((p.K, B))
+
+
 def _episodes_setup_context(ctx, inputs, output):
     robot_init, plan_weights, weight_idx, true_weights, unlucky_idx, params, scenario, T = inputs
     ctx.save_for_backward(robot_init, plan_weights, weight_idx, true_weights, unlucky_idx)
@@ -228,9 +253,11 @@ def _episodes_backward(ctx, returns_bar):
     # the trace of the forward's own run: the same kernel on the same inputs, so the same bits
     _, controls, best, states = torch.ops.ocd_b200.episodes_trace(robot_init, plan_weights, weight_idx, true_weights,
                                                                   unlucky_idx, ctx.params, ctx.scenario, ctx.T)
-    pw_bar, ri_bar, tw_bar = torch.ops.ocd_b200.episodes_vjp(plan_weights, weight_idx, true_weights, states, best,
-                                                            controls, returns_bar.contiguous(), ctx.params,
-                                                            ctx.scenario, ctx.T)
+    # L-BFGS: the implicit-function derivative of every step's optimum (the line search is not differentiated)
+    vjp = torch.ops.ocd_b200.episodes_implicit_vjp if unpack_params(ctx.params).optimizer == 1 \
+        else torch.ops.ocd_b200.episodes_vjp
+    pw_bar, ri_bar, tw_bar = vjp(plan_weights, weight_idx, true_weights, states, best, controls,
+                                 returns_bar.contiguous(), ctx.params, ctx.scenario, ctx.T)
     Bw, B = plan_weights.shape[-1], robot_init.shape[-1]
     if weight_idx is not None:
         # rows of the worlds that share a vector, summed deterministically (see _solve_backward)
